@@ -13,15 +13,21 @@ reported alongside.  Other BASELINE configs: --workload c1 | c2 | c4.
 
     python bench.py --gpus N --steps K --warmup W            # B200 arm
     python bench.py --impl reference ...                     # CPU oracle arm
+    python bench.py --dump-outputs DIR ...                   # also write the last timed step's results
+
+The run writes nothing into the source tree: kernels and model code it compiles go to a temporary
+directory (kernel sets that __graft_entry__.build() prebuilt are read from the tree).
 """
 import argparse
 import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
+sys.dont_write_bytecode = True
 ROOT = os.path.dirname(os.path.abspath(__file__))
 for p in (ROOT, os.path.join(ROOT, "oracle")):
     if p not in sys.path:
@@ -108,7 +114,14 @@ def parse():
     ap.add_argument("--lanes", type=int, default=0, help="debug: override lane count")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--workload", default="c3", choices=sorted(WORKLOADS))
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (float64, at most 64 MB)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the results of the B200 arm")
+    return args
 
 
 class ClockSampler:
@@ -290,6 +303,27 @@ def run_reference(args):
     print(json.dumps(line), flush=True)
 
 
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(path, u, t, st, adaptive):
+    """--dump-outputs: what the sweep's caller receives from the last timed step, as <path>/<name>.npy in float64.
+    u [save][T][P] waveforms and t ([T], or [T][P] when adaptive) come for a fixed, seeded sample of lanes
+    (lanes.npy) sized so that all files stay within DUMP_BYTES; status, newton_iters and count (saved points)
+    come for every lane.  Adaptive waveforms are zero past a lane's count."""
+    os.makedirs(path, exist_ok=True)
+    n_save, T, P = u.shape
+    budget = DUMP_BYTES - 4096 - 8 * 3 * P - (0 if adaptive else 8 * T)          # 4096: the .npy headers
+    k = int(min(P, budget // (8 * (T * (n_save + adaptive) + 1))))
+    lanes = np.arange(P) if k == P else np.sort(np.random.default_rng(0).choice(P, k, replace=False))
+    valid = np.arange(T)[:, None] < st[2, lanes][None, :]
+    out = {"lanes": lanes, "status": st[0], "newton_iters": st[1], "count": st[2],
+           "u": np.where(valid[None], u[:, :, lanes], 0.0),
+           "t": np.where(valid, t[:, lanes], 0.0) if adaptive else t}
+    for name, a in out.items():
+        np.save(os.path.join(path, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def run_b200(args):
     import torch
     import torch.distributed as dist
@@ -345,7 +379,7 @@ def run_b200(args):
     # 30 inlined model instances are beyond a straight-line kernel: C4 runs table-driven
     use_spec = os.environ.get("CB200_NO_SPECIALIZE", "0") != "1" and not adaptive
     if use_spec:
-        comp.specialize(DT, "be", limit=W["limit"], fixed_only=True)        # emitter: circuit-specialised kernels (nvcc, cached in-tree)
+        comp.specialize(DT, "be", limit=W["limit"], fixed_only=True)        # emitter: circuit-specialised kernels (nvcc)
 
     def tran_resident():
         if adaptive:
@@ -402,13 +436,25 @@ def run_b200(args):
     t0 = time.perf_counter()
     kern_ms = tran_ms = 0.0
     launches = 0
-    for _ in range(args.steps):
+    last_wave = None
+    for i in range(args.steps):
         wave, st = step_resident()
         kern_ms += st["kernel_ms"]; tran_ms += st["tran_kernel_ms"]; launches += st["launches"]
-        wave.free()
+        if args.dump_outputs and i == args.steps - 1:
+            last_wave = wave                 # fetched after the timed region
+        else:
+            wave.free()
         flush.zero_()
     barrier()
     wall = time.perf_counter() - t0
+    if last_wave is not None:                # every rank's block of the sweep into the shared host arrays
+        r = last_wave.fetch(out_np, t_full.lane_block(sl) if adaptive else None)
+        last_wave.free()
+        st_full.array[0, sl] = r["status"]; st_full.array[1, sl] = r["newton_iters"]; st_full.array[2, sl] = r["count"]
+        barrier()
+        if rank == 0:
+            dump_outputs(args.dump_outputs, out_full.array, t_full.array if adaptive else r["t"], st_full.array,
+                         adaptive)
     # ---- timed: end to end through the C ABI with host buffers; ends when every rank's block of
     # the full-sweep waveform array is in host memory (the final gather) -------
     barrier()
@@ -674,10 +720,15 @@ def c1_eval_times(cb, backend):
 def main():
     args = parse()
     select_workload(args.workload)
-    if args.impl == "reference":
-        run_reference(args)
-    else:
-        run_b200(args)
+    import cadnip_oracle as ora
+    from cadnip_b200 import backend
+    with tempfile.TemporaryDirectory(prefix="cadnip_b200_bench_") as cache:
+        backend.RUN_CACHE_DIR = os.path.join(cache, "kernels")
+        ora.GEN_DIR = os.path.join(cache, "oracle")
+        if args.impl == "reference":
+            run_reference(args)
+        else:
+            run_b200(args)
 
 
 if __name__ == "__main__":

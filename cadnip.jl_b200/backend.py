@@ -25,6 +25,9 @@ _SOURCES = ["api.cu", "kernels.cu", "symbolic.cpp", "specialize.cpp"]
 _HEADERS = ["kernels.h", "cb200_internal.h", "lane_kernels.cuh", "warp_kernels.cuh", "group_kernels.inc", "specialize.h",
             os.path.join("..", "..", "include", "cadnip_b200.h")]
 GEN_DIR = os.path.join(_HERE, "_gen")
+# Kernels compiled at run time (circuit-specialised kernels, kernel sets that GEN_DIR does not hold yet) are
+# cached here.  A caller that must leave the tree untouched points it at a directory of its own.
+RUN_CACHE_DIR = GEN_DIR
 
 OK, EINVAL, ENOMEM, ECUDA, ENODEVICE, ESTATE, ESINGULAR = 0, -1, -2, -3, -4, -5, -6
 LANE_OK, LANE_MAXITER, LANE_SINGULAR, LANE_NONFINITE, LANE_DTMIN = 0, 1, 2, 3, 4
@@ -481,7 +484,8 @@ class Handle:
 
     def load_va_models(self, cuda_header: str):
         """Rebuild (cached) and load the kernel set with the circuit's Verilog-A models."""
-        self._check(lib().cb200_load_va_models(self._p, cuda_header.encode(), _CSRC.encode(), GEN_DIR.encode()))
+        cache = GEN_DIR if va_models_cached(cuda_header) else RUN_CACHE_DIR
+        self._check(lib().cb200_load_va_models(self._p, cuda_header.encode(), _CSRC.encode(), cache.encode()))
 
     def _check(self, rc: int):
         if rc != OK:
@@ -530,13 +534,13 @@ class Handle:
 
     def specialize(self, spec: MNASpec, method, dt: float, compile_only: bool = False, limit: bool = False,
                    fixed_only: bool = False):
-        """Generate + compile (cached in cadnip.jl_b200/_gen) + load kernels specialised
+        """Generate + compile (cached in RUN_CACHE_DIR) + load kernels specialised
         for this circuit; later dc/tran calls use them.  limit: include the CB200_TRAN_LIMIT
         path (otherwise transients that ask for it run on the table-driven kernels)."""
         s = make_spec(spec, "tran")
         m = METHODS[method] if isinstance(method, str) else int(method)
         self._check(lib().cb200_specialize(self._p, C.byref(s), m, float(dt), _CSRC.encode(),
-                                           GEN_DIR.encode(), (1 if compile_only else 0) | (2 if limit else 0) | (4 if fixed_only else 0)))
+                                           RUN_CACHE_DIR.encode(), (1 if compile_only else 0) | (2 if limit else 0) | (4 if fixed_only else 0)))
 
     def is_specialized(self) -> bool:
         return bool(lib().cb200_is_specialized(self._p))

@@ -15,6 +15,8 @@ import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _LIB_PATH = os.path.join(_HERE, "libcadnip_oracle.so")
+# cache of the compiled Verilog-A model code; a caller that must leave the tree untouched points it elsewhere
+GEN_DIR = os.path.join(_HERE, "_gen")
 
 
 def build(force: bool = False) -> str:
@@ -345,7 +347,7 @@ _va_libs = []
 
 def load_va_models(models, count_ops: bool = False) -> None:
     """Compile the C the product's emitter generated for these Verilog-A modules
-    (gcc, cached under oracle/_gen) and register it with the oracle.  The model index
+    (gcc, cached under GEN_DIR) and register it with the oracle.  The model index
     is the position in ``models`` (== dev_flags of the lowered circuit).
     count_ops: build the op-counting variant (verilog_a.instrument_ops) -- `va_op_counts()` then
     returns the flops / transcendentals the model code EXECUTED since `va_op_reset()`; counting
@@ -363,12 +365,11 @@ def load_va_models(models, count_ops: bool = False) -> None:
         sys.path.insert(0, os.path.dirname(_HERE))
         import cadnip_b200.verilog_a as va
         src = va.instrument_ops(src)
-    gen = os.path.join(_HERE, "_gen")
-    os.makedirs(gen, exist_ok=True)
+    os.makedirs(GEN_DIR, exist_ok=True)
     h = hashlib.sha256(src.encode()).hexdigest()[:16]
-    so = os.path.join(gen, f"va_{h}.so")
+    so = os.path.join(GEN_DIR, f"va_{h}.so")
     if not os.path.exists(so):
-        cfile = os.path.join(gen, f"va_{h}.c")
+        cfile = os.path.join(GEN_DIR, f"va_{h}.c")
         with open(cfile, "w") as f:
             f.write(src)
         cc = "/usr/bin/gcc" if os.path.exists("/usr/bin/gcc") else "gcc"

@@ -428,9 +428,26 @@ def test_emitted_model_matches_interpreter(name, kw, bias):
     differentiation.  One instance with every port on a voltage source, internal nodes at random voltages,
     limit unknowns on their probe voltages: the KCL rows of G u - b must equal the interpreter's branch
     currents, and the stamped G must equal central differences OF THE INTERPRETER."""
-    from cadnip_b200 import verilog_a, MNAContext, ZERO_VECTOR, stamp, VoltageSource
+    from cadnip_b200 import verilog_a
     import va_circuits
-    m = verilog_a.load_va(va_circuits.VA_DIR + name + ".va")
+    _check_against_interpreter(verilog_a.load_va(va_circuits.VA_DIR + name + ".va"), kw, bias)
+
+
+INLINE_INTERP_CASES = [("VADDiode", [0.65, 0.05]), ("VADDiodeRs", [0.65, 0.05]), ("ChainDiodeRs", [0.7, 0.0]),
+                       ("SimpleMOS", [1.5, 1.2, 0.1]), ("CapMOS", [1.5, 1.2, 0.1]), ("PMOS", [0.1, 0.2, 1.5]),
+                       ("JunctionCap", [-0.5, 0.0])]
+
+
+@pytest.mark.parametrize("name,bias", INLINE_INTERP_CASES, ids=[c[0] for c in INLINE_INTERP_CASES])
+def test_inline_model_matches_interpreter(name, bias):
+    """The same emitter-independent check on the Verilog-A modules written out in tests/test_va.py, so that it
+    runs wherever the repository does."""
+    import test_va
+    _check_against_interpreter(getattr(test_va, name), {}, bias)
+
+
+def _check_against_interpreter(m, kw, bias):
+    from cadnip_b200 import MNAContext, ZERO_VECTOR, stamp, VoltageSource
     held = {}
 
     def builder(params, spec, t=0.0, x=ZERO_VECTOR, ctx=None):
@@ -481,7 +498,7 @@ def test_emitted_model_matches_interpreter(name, kw, bias):
     I_int = interp(u)
     assert np.all(np.isfinite(I_emit)) and np.all(np.isfinite(Gd))
     scale = max(float(np.abs(I_int).max()), 1e-30)
-    assert np.max(np.abs(I_emit - I_int)) <= 1e-9 * scale, (name, I_emit, I_int)
+    assert np.max(np.abs(I_emit - I_int)) <= 1e-9 * scale, (m.name, I_emit, I_int)
     gs = float(np.abs(Gd[:lc.n_nodes, :lc.n_nodes]).max()) + 1e-30
     for j in range(lc.n_nodes):
         h = 1e-6
@@ -491,7 +508,7 @@ def test_emitted_model_matches_interpreter(name, kw, bias):
         col = Gd[:lc.n_nodes, j].copy()
         for k, (p, q) in enumerate(lim):                     # limit unknowns follow their probes
             col += Gd[:lc.n_nodes, n - lc.n_limits + k] * ((1.0 if p == j + 1 else 0.0) - (1.0 if q == j + 1 else 0.0))
-        assert np.max(np.abs(dI - col)) <= 1e-6 * gs, (name, j, float(np.max(np.abs(dI - col)) / gs))
+        assert np.max(np.abs(dI - col)) <= 1e-6 * gs, (m.name, j, float(np.max(np.abs(dI - col)) / gs))
 
 
 def lc_limit_branches(lc):
