@@ -1148,7 +1148,7 @@ static int tran_impl(cb200_handle *h, const cb200_spec *spec, double t0, double 
     if (ce != cudaSuccess) { delete w; return fail(h, CB200_ECUDA, cudaGetErrorString(ce)); }
     if (!o->adaptive) h->stats.steps_accepted = w->nsteps * P;
     if (!o->adaptive && used_spec && h->spec.take_counters) {
-        // specialised kernels skip quiescent steps bit-exactly (specialize.cpp, kSpecTranFixedBody): the
+        // specialised kernels skip quiescent steps bit-exactly (lane_kernels.cuh, tran_fixed_body): the
         // lane-steps actually executed
         unsigned long long nexec = 0;
         if (h->spec.take_counters(&nexec, s) == cudaSuccess) h->stats.steps_accepted = (int64_t)nexec;
@@ -1244,6 +1244,29 @@ extern "C" int cb200_set_tstops(cb200_handle *h, const double *tstops, int32_t n
 // ---------------------------------------------------------------------------
 // circuit specialisation (the emitter)
 // ---------------------------------------------------------------------------
+// What the emitter reads of a handle's circuit, and the launch bounds of the generated kernels: 64 threads
+// per block and enough resident blocks per SM for all P lanes in one wave, as far as registers allow.
+static SpecInput spec_input(const cb200_handle &h, int method, int64_t P, int num_sms)
+{
+    SpecInput in{};
+    in.st = &h.st; in.prog = &h.prog;
+    in.dev_kind = &h.dev_kind; in.dev_flags = &h.dev_flags; in.dev_node_ptr = &h.dev_node_ptr;
+    in.dev_nodes = &h.dev_nodes; in.dev_param_ptr = &h.dev_param_ptr; in.dev_params = &h.dev_params;
+    in.dev_gbase = &h.dev_gbase; in.dev_cbase = &h.dev_cbase; in.dev_bbase = &h.dev_bbase; in.dev_sbase = &h.dev_sbase;
+    in.src_list = &h.src_list; in.nl_list = &h.nl_list; in.limit_init_ref = &h.limit_init_ref;
+    in.src_uniform = &h.src_uniform; in.method = method;
+    in.va_header_path = h.k.va_header_path;
+    in.uniform = &h.uniform; in.lu_dc = &h.lu[0].host; in.lu_tr = &h.lu[1].host;
+    in.n_lane_cols = h.n_lane_cols;
+    in.block = 64;
+    const int64_t lanes_per_sm = (P + num_sms - 1) / num_sms;
+    in.min_blocks = std::max(1, std::min((int)((lanes_per_sm + in.block - 1) / in.block), 1024 / in.block));
+    // a lane state beyond the register file lives in local memory: measured on B200 (C3, sp_mos1
+    // inverter, 432 slots) 4 resident blocks x 255 registers beat 11 x 93 by 1.6x
+    if (h.prog.n_slots > 120) in.min_blocks = std::min(in.min_blocks, 4);
+    return in;
+}
+
 extern "C" int cb200_specialize(cb200_handle *h, const cb200_spec *spec, int32_t method, double dt,
                                 const char *csrc_dir, const char *cache_dir, int32_t flags)
 {
@@ -1261,31 +1284,9 @@ extern "C" int cb200_specialize(cb200_handle *h, const cb200_spec *spec, int32_t
     const bool want_adaptive = (flags & CB200_SPEC_FIXED_ONLY) == 0;
     if (spec_usable(h) && h->spec_method == method && h->spec_limit == want_limit &&
         (!want_adaptive || h->spec.tran_adaptive)) return CB200_OK;
-    SpecInput in{};
+    SpecInput in = spec_input(*h, method, h->P, h->num_sms);
     in.tran_limit = want_limit;
     in.with_adaptive = want_adaptive;
-    in.st = &h->st; in.prog = &h->prog;
-    in.dev_kind = &h->dev_kind; in.dev_flags = &h->dev_flags; in.dev_node_ptr = &h->dev_node_ptr;
-    in.dev_nodes = &h->dev_nodes; in.dev_param_ptr = &h->dev_param_ptr; in.dev_params = &h->dev_params;
-    in.dev_gbase = &h->dev_gbase; in.dev_cbase = &h->dev_cbase; in.dev_bbase = &h->dev_bbase; in.dev_sbase = &h->dev_sbase;
-    in.src_list = &h->src_list; in.nl_list = &h->nl_list; in.limit_init_ref = &h->limit_init_ref;
-    in.src_uniform = &h->src_uniform; in.method = method;
-    in.va_header_path = h->k.va_header_path;
-    in.uniform = &h->uniform; in.lu_dc = &h->lu[0].host; in.lu_tr = &h->lu[1].host;
-    in.n_lane_cols = h->n_lane_cols;
-    // one wave: enough resident blocks per SM for all lanes, as far as registers allow
-    in.block = 64;
-    const int64_t lanes_per_sm = (h->P + h->num_sms - 1) / h->num_sms;
-    int mb = (int)((lanes_per_sm + in.block - 1) / in.block);
-    in.min_blocks = std::max(1, std::min(mb, 1024 / in.block));
-    // a lane state beyond the register file lives in local memory: measured on B200 (C3, sp_mos1
-    // inverter, 432 slots) 4 resident blocks x 255 registers beat 11 x 93 by 1.6x
-    if (h->prog.n_slots > 120) in.min_blocks = std::min(in.min_blocks, 4);
-    if (const char *e = getenv("CB200_SPEC_MINBLOCKS")) in.min_blocks = std::max(1, atoi(e));   // tuning knob
-    if (getenv("CB200_LOCKSTEP")) {                // experiment: one block of 8 lockstep warps per SM (specialize.cpp)
-        in.block = getenv("CB200_SPEC_BLOCK") ? std::max(32, atoi(getenv("CB200_SPEC_BLOCK"))) : 256;
-        in.min_blocks = 1;
-    }
     if (h->prog.n_slots > 4096) return fail(h, CB200_EINVAL, "cb200_specialize: circuit too large for a register-resident kernel");
     const std::string src = generate_spec_source(in);
     unload_spec(h->spec);
@@ -1413,19 +1414,7 @@ extern "C" int64_t cb200_emit_source(const cb200_desc *d, const double *absJ_dc,
     if (e.empty()) e = analyze_lu(h.st, a1, 1e-3, h.lu[1].host);
     if (!e.empty()) { g_last_error = e; return CB200_ESINGULAR; }
     layout_workspace(&h);
-    SpecInput in{};
-    in.st = &h.st; in.prog = &h.prog;
-    in.dev_kind = &h.dev_kind; in.dev_flags = &h.dev_flags; in.dev_node_ptr = &h.dev_node_ptr;
-    in.dev_nodes = &h.dev_nodes; in.dev_param_ptr = &h.dev_param_ptr; in.dev_params = &h.dev_params;
-    in.dev_gbase = &h.dev_gbase; in.dev_cbase = &h.dev_cbase; in.dev_bbase = &h.dev_bbase; in.dev_sbase = &h.dev_sbase;
-    in.src_list = &h.src_list; in.nl_list = &h.nl_list; in.limit_init_ref = &h.limit_init_ref;
-    in.src_uniform = &h.src_uniform; in.method = method;
-    in.uniform = &h.uniform; in.lu_dc = &h.lu[0].host; in.lu_tr = &h.lu[1].host;
-    in.n_lane_cols = h.n_lane_cols;
-    in.block = 64;
-    const int64_t lanes_per_sm = (P + num_sms - 1) / num_sms;
-    in.min_blocks = std::max(1, std::min((int)((lanes_per_sm + in.block - 1) / in.block), 1024 / in.block));
-    if (h.prog.n_slots > 120) in.min_blocks = std::min(in.min_blocks, 4);
+    const SpecInput in = spec_input(h, method, P, num_sms);
     const std::string src = generate_spec_source(in);
     if (out && cap > 0) {
         const int64_t m = std::min<int64_t>(cap - 1, (int64_t)src.size());

@@ -93,7 +93,7 @@ struct DcArgs {
     unsigned char *converged;  // [P]
     int *weak;              // [P] or null: set to 1 when a refactor of the lane met a weak pivot (see weak_pivot())
     double *ws_global;      // used when the lane workspace does not fit in shared memory
-    int hot_smem;           // set by the launcher (lane-per-warp kernels: shared-memory configuration)
+    int gather_ch;          // set by the launcher: doubles of the shared-memory gather buffer of a lane-per-warp / -block lane
 };
 cudaError_t launch_dc(const Program &p, const LuProgram &lu, const SpecArgs &s, const DcArgs &a,
                       int block, size_t smem_limit, cudaStream_t st, int64_t *launches);
@@ -120,7 +120,7 @@ struct TranArgs {
     int *evals;             // [P] or null: += device-model evaluation passes executed for the lane
     int *weak;              // [P] or null (see DcArgs)
     double *ws_global;
-    int hot_smem;
+    int gather_ch;
 };
 cudaError_t launch_tran_fixed(const Program &p, const LuProgram &lu, const SpecArgs &s,
                               const TranArgs &a, int block, size_t smem_limit, cudaStream_t st,
@@ -150,7 +150,7 @@ struct AdaptArgs {
     int *evals;             // [P] or null (see TranArgs)
     int *weak;              // [P] or null (see DcArgs)
     double *ws_global;
-    int hot_smem;
+    int gather_ch;
 };
 cudaError_t launch_tran_adaptive(const Program &p, const LuProgram &lu, const SpecArgs &s,
                                  const AdaptArgs &a, int block, size_t smem_limit,

@@ -44,6 +44,7 @@ struct DynProg {
     static constexpr int kUnroll = 1;
     static constexpr int kMethod = -1;      // integration method chosen at run time
     static constexpr bool kTranLimit = true; // CB200_TRAN_LIMIT supported (specialised kernels: opt-in)
+    static constexpr bool kBypass = false;   // quiescent-step bypass of tran_fixed_body (generated programs only)
     const Program &p;
     __device__ __forceinline__ explicit DynProg(const Program &pp) : p(pp) {}
     __device__ __forceinline__ int n() const { return p.n; }
@@ -979,13 +980,69 @@ __device__ __forceinline__ void dc_stepping_body(const PG &pg, const LU &lu, W &
 }
 
 // ---------------------------------------------------------------------------
+// Newton iteration of one implicit step (both transient bodies), from the predictor in u: rebuild,
+// F, stop when ||F||_2 < abstol, otherwise solve J delta = F and update; at most max_nl solves.
+// Masked: a lane that is done (`done` on entry: a lane that has finished its time loop) keeps its
+// state but still takes part in the warp's evaluations, solves and votes.
+// `limit` (CB200_TRAN_LIMIT): a step the plain iteration does not finish in max_nl solves is redone
+// from u_n with the PCNR corrector after every solve (4*max_nl solves allowed); lim_on reports it.
+// Returns the CB200_LANE_* status of the step.  Counts solves and evaluation passes; `fresh`: see
+// tran_fixed_body.
+// ---------------------------------------------------------------------------
+template <typename PG, typename LU, typename W>
+__device__ __forceinline__ int newton_step(const PG &pg, const LU &lu, W &w, const SpecArgs &sp, bool done,
+                                           double t, double gamma, double abstol2, int max_nl, int limit,
+                                           int &solves, int &evals, bool &fresh, bool &lim_on)
+{
+    int st = CB200_LANE_OK;
+    lim_on = false;
+    int it0 = 0;
+    for (int it = 0;; it++) {
+        // lanes that are fresh recompute identical values when another lane of the warp is not
+        if (__any_sync(0xffffffffu, kNlTimeDep || !fresh)) { eval_nonlinear(pg, w, t, CB200_MODE_TRAN, false); evals++; }
+        fresh = true;
+        bool bad;
+        const double nrm2 = assemble<true>(pg, lu, w, gamma, sp.gshunt, sp.srcFact, bad);
+        bool restart = false;
+        if (!done) {
+            if (bad) { done = true; st = CB200_LANE_NONFINITE; }
+            else if (nrm2 < abstol2) { done = true; }
+            else if (it - it0 >= (lim_on ? 4 * max_nl : max_nl)) {
+                if (PG::kTranLimit && limit && !lim_on) { lim_on = true; it0 = it + 1; restart = true; }
+                else { done = true; st = CB200_LANE_MAXITER; }
+            }
+        }
+        if (__all_sync(0xffffffffu, done)) break;
+        bool singular;
+        const bool ok = factor_and_solve(pg, lu, w, singular);
+        if (!done) {
+            if (restart) {                             // redo the step from u_n, limiting on
+                CB_UNROLL
+                for (int i = 0; i < pg.n(); i++) w(pg.off_u() + i) = w(pg.off_un() + i);
+                fresh = false;
+            } else if (!ok) { done = true; st = singular ? CB200_LANE_SINGULAR : CB200_LANE_NONFINITE; }
+            else {
+                apply_update(pg, lu, w);
+                fresh = false;
+                solves++;
+                if (lim_on) {                          // PCNR corrector, solve.jl:686-689
+                    const int lim0 = pg.n() - pg.n_limits();
+                    CB_UNROLL
+                    for (int q = 0; q < pg.n_limits(); q++) w(pg.off_u() + lim0 + q) = w(pg.off_limw() + q);
+                }
+            }
+        }
+    }
+    return st;
+}
+
+// ---------------------------------------------------------------------------
 // fixed-step transient body: the whole time loop of a lane on the device.
 //   du = gamma*(u - u_n) + dterm
 //   BE:    gamma = 1/h,      dterm = 0
 //   trap:  gamma = 2/h,      dterm = -du_n                      (first step BE)
 //   Gear2: gamma = 3/(2h),   dterm = -(u_n - u_{n-1})/(2h)      (first step BE)
-// Newton per step from u = u_n: rebuild, F, stop when ||F||_2 < abstol, otherwise
-// solve J delta = F and update; at most max_nl solves.  t_k = t0 + k*h.
+// Newton per step from u = u_n (newton_step).  t_k = t0 + k*h.
 // ---------------------------------------------------------------------------
 template <typename PG, typename LU, typename W>
 __device__ __forceinline__ void tran_fixed_body(const PG &pg, const LU &lu, W &w, const Program &p,
@@ -1027,11 +1084,38 @@ __device__ __forceinline__ void tran_fixed_body(const PG &pg, const LU &lu, W &w
     // u alone, so the first residual of a step re-assembles them with the new source values and
     // history terms instead of evaluating every device model again for identical values.
     bool fresh = false;
+    // Quiescent-step bypass (PG::kBypass, backward Euler; a generated program knows its source stamp slots at
+    // compile time).  `quiet`: the previous step of this lane converged at its first residual -- no solve, so
+    // u == u_n, d == 0 and the stamps are those of u.  If in addition every source stamp of the new step is
+    // bitwise what it was, the new step's first residual F = G u - b is bit for bit the one that just passed
+    // the test: the step would assemble the same numbers, find them converged and change nothing.  When that
+    // holds for all 32 lanes of the warp the step is not executed (its saved point is written from the
+    // unchanged u).  Identical waveforms, statuses and Newton counts by construction; a lane that could not
+    // skip alone executes the step as usual.
+    bool quiet = false;
+    int nexec = 0;                                 // steps this lane executed (not bypassed)
     for (int64_t k = a.k_begin; k <= a.k_end; k++) {
         const double t = a.t0 + (double)k * h;
         const int method = (k == 1) ? CB200_METHOD_BE : amethod;
         const double gamma = method == CB200_METHOD_BE ? 1.0 / h
                            : method == CB200_METHOD_TRAP ? 2.0 / h : 3.0 / (2.0 * h);
+        if constexpr (PG::kBypass) {
+            double src_old[PG::kSrcSlots > 0 ? PG::kSrcSlots : 1];
+            PG::src_snapshot(w, src_old);
+            eval_sources_step(pg, w, k, k == a.k_begin, a.t0, h, CB200_MODE_TRAN);
+            if (PG::kMethod == CB200_METHOD_BE && !kNlTimeDep) {
+                if (__all_sync(0xffffffffu, PG::src_same(w, src_old, quiet && k != a.k_begin))) {
+                    if (k % a.save_every == 0 || k == a.nsteps) {
+                        if (act)
+                            for (int q = 0; q < a.n_save; q++)
+                                a.out[((int64_t)q * a.T + tp) * p.P + lane] = read_u(pg, w, __ldg(a.save_idx + q));
+                        tp++;
+                    }
+                    continue;
+                }
+            }
+            nexec++;
+        }
         // history terms; un <- u
         CB_UNROLL
         for (int i = 0; i < pg.n(); i++) {
@@ -1041,49 +1125,14 @@ __device__ __forceinline__ void tran_fixed_body(const PG &pg, const LU &lu, W &w
             /* trap: dterm already holds -du_n */
             w(pg.off_un() + i) = ui;
         }
-        eval_sources_step(pg, w, k, k == a.k_begin, a.t0, h, CB200_MODE_TRAN);
-        bool done = false;
-        int st = CB200_LANE_OK;
-        // a.limit (CB200_TRAN_LIMIT): a step the plain iteration does not finish in max_nl solves
-        // is redone from u_n with the PCNR corrector after every solve (4*max_nl solves allowed)
-        bool lim_on = false;
-        int it0 = 0;
-        for (int it = 0;; it++) {
-            // lanes that are fresh recompute identical values when another lane of the warp is not
-            if (__any_sync(0xffffffffu, kNlTimeDep || !fresh)) { eval_nonlinear(pg, w, t, CB200_MODE_TRAN, false); evals++; }
-            fresh = true;
-            bool bad;
-            const double nrm2 = assemble<true>(pg, lu, w, gamma, sp.gshunt, sp.srcFact, bad);
-            bool restart = false;
-            if (!done) {
-                if (bad) { done = true; st = CB200_LANE_NONFINITE; }
-                else if (nrm2 < abstol2) { done = true; }
-                else if (it - it0 >= (lim_on ? 4 * a.max_nl : a.max_nl)) {
-                    if (PG::kTranLimit && a.limit && !lim_on) { lim_on = true; it0 = it + 1; restart = true; }
-                    else { done = true; st = CB200_LANE_MAXITER; }
-                }
-            }
-            if (__all_sync(0xffffffffu, done)) break;
-            bool singular;
-            const bool ok = factor_and_solve(pg, lu, w, singular);
-            if (!done) {
-                if (restart) {                             // redo the step from u_n, limiting on
-                    CB_UNROLL
-                    for (int i = 0; i < pg.n(); i++) w(pg.off_u() + i) = w(pg.off_un() + i);
-                    fresh = false;
-                } else if (!ok) { done = true; st = singular ? CB200_LANE_SINGULAR : CB200_LANE_NONFINITE; }
-                else {
-                    apply_update(pg, lu, w);
-                    fresh = false;
-                    solves++;
-                    if (lim_on) {                          // PCNR corrector, solve.jl:686-689
-                        const int lim0 = pg.n() - pg.n_limits();
-                        CB_UNROLL
-                        for (int q = 0; q < pg.n_limits(); q++) w(pg.off_u() + lim0 + q) = w(pg.off_limw() + q);
-                    }
-                }
-            }
-        }
+        // with the bypass the sources were evaluated above, where it tests them; both orders give the same
+        // results, and here the table-driven kernels keep the register allocation they were measured with
+        if constexpr (!PG::kBypass) eval_sources_step(pg, w, k, k == a.k_begin, a.t0, h, CB200_MODE_TRAN);
+        const int solves0 = solves;
+        bool lim_on;
+        const int st = newton_step(pg, lu, w, sp, false, t, gamma, abstol2, a.max_nl, a.limit, solves, evals, fresh,
+                                   lim_on);
+        quiet = st == CB200_LANE_OK && solves == solves0 && !lim_on;
         if (st != CB200_LANE_OK && status == CB200_LANE_OK) status = st;
         if (st != CB200_LANE_OK) fresh = false;           // the last evaluation was not at the state kept
         if (st == CB200_LANE_NONFINITE || st == CB200_LANE_SINGULAR) {  // dead lane: hold last state
@@ -1115,6 +1164,7 @@ __device__ __forceinline__ void tran_fixed_body(const PG &pg, const LU &lu, W &w
         if (a.weak && w.weak) a.weak[lane] = 1;
         a.iters[lane] += solves;
         if (a.evals != nullptr) a.evals[lane] += evals;
+        if constexpr (PG::kBypass) PG::count_steps(nexec);
     }
 }
 
@@ -1426,47 +1476,9 @@ __device__ __forceinline__ void tran_adaptive_body(const PG &pg, const LU &lu, W
         }
         eval_sources(pg, w, tn, CB200_MODE_TRAN);
         // ---- Newton on the implicit step
-        bool done = finished;
-        int st = CB200_LANE_OK;
-        // a.limit (CB200_TRAN_LIMIT): a step the plain iteration does not finish in max_nl solves
-        // is redone from u_n with the PCNR corrector after every solve (4*max_nl solves allowed)
-        bool lim_on = false;
-        int it0 = 0;
-        for (int it = 0;; it++) {
-            if (__any_sync(0xffffffffu, kNlTimeDep || !fresh)) { eval_nonlinear(pg, w, tn, CB200_MODE_TRAN, false); evals++; }
-            fresh = true;
-            bool bad;
-            const double nrm2 = assemble<true>(pg, lu, w, gamma, sp.gshunt, sp.srcFact, bad);
-            bool restart = false;
-            if (!done) {
-                if (bad) { done = true; st = CB200_LANE_NONFINITE; }
-                else if (nrm2 < abstol2) { done = true; }
-                else if (it - it0 >= (lim_on ? 4 * a.max_nl : a.max_nl)) {
-                    if (PG::kTranLimit && a.limit && !lim_on) { lim_on = true; it0 = it + 1; restart = true; }
-                    else { done = true; st = CB200_LANE_MAXITER; }
-                }
-            }
-            if (__all_sync(0xffffffffu, done)) break;
-            bool singular;
-            const bool ok = factor_and_solve(pg, lu, w, singular);
-            if (!done) {
-                if (restart) {                             // redo the step from u_n, limiting on
-                    CB_UNROLL
-                    for (int i = 0; i < pg.n(); i++) w(pg.off_u() + i) = w(pg.off_un() + i);
-                    fresh = false;
-                } else if (!ok) { done = true; st = singular ? CB200_LANE_SINGULAR : CB200_LANE_NONFINITE; }
-                else {
-                    apply_update(pg, lu, w);
-                    fresh = false;
-                    solves++;
-                    if (lim_on) {                          // PCNR corrector, solve.jl:686-689
-                        const int lim0 = pg.n() - pg.n_limits();
-                        CB_UNROLL
-                        for (int q = 0; q < pg.n_limits(); q++) w(pg.off_u() + lim0 + q) = w(pg.off_limw() + q);
-                    }
-                }
-            }
-        }
+        bool lim_on;
+        const int st = newton_step(pg, lu, w, sp, finished, tn, gamma, abstol2, a.max_nl, a.limit, solves, evals, fresh,
+                                   lim_on);
         if (finished) continue;
         if (bdf) {
             bool fail = st != CB200_LANE_OK;

@@ -201,263 +201,26 @@ static void emit_lu(std::ostringstream &o, const char *sname, const Structure &s
     o << "};\n";
 }
 
-// ---------------------------------------------------------------------------
-// The fixed-step time loop of the SPECIALISED kernels: tran_fixed_body of lane_kernels.cuh, statement for
-// statement, plus the quiescent-step bypass described in the text below (a circuit-specialised kernel knows
-// its source stamp slots at compile time, which is what the test needs).  The table-driven kernels keep the
-// plain loop; both produce identical results (tests/test_gpu_parity.py: specialised vs table-driven vs oracle).
-// @SRC_OLD@ / @SRC_SAME@ are filled per circuit; CB200_NO_BYPASS=1 generates kernels on the plain loop.
-// ---------------------------------------------------------------------------
-static const char *kSpecTranFixedBody = R"CB200(
-template <typename PG, typename LU, typename W>
-__device__ __forceinline__ void spec_tran_fixed_body(const PG &pg, const LU &lu, W &w, const Program &p,
-                                                const SpecArgs &sp, const TranArgs &a)
-{
-    const int64_t lane0 = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    const bool act = lane0 < p.P;
-    const int64_t lane = act ? lane0 : p.P - 1;
-
-    // The time loop may be cut into segments [k_begin, k_end] (one launch each) so that the
-    // copy of a finished segment's waveform to the host overlaps the next segment's compute;
-    // a resumed segment reloads the integrator history (u_n, dterm) the previous one stored.
-    const bool resume = a.k_begin > 1;
-    load_lane_params(pg, w, p.lanes, p.P, lane);
-    CB_UNROLL
-    for (int i = 0; i < pg.n(); i++) {
-        w(pg.off_u() + i) = a.u[(int64_t)i * p.P + lane];
-        w(pg.off_dterm() + i) = resume ? a.hist[(int64_t)(pg.n() + i) * p.P + lane] : 0.0;
-        w(pg.off_un() + i) = resume ? a.hist[(int64_t)i * p.P + lane] : 0.0;
-    }
-    eval_all(pg, w, a.t0, CB200_MODE_TRAN, false);
-
-    int status = a.status[lane], solves = 0;       // keeps an InitialFailure from the DC init
-    int evals = 0;                                 // device-model evaluation passes this thread executed
-    int64_t tp = a.tp_begin;
-    if (!resume) {
-        if (act)
-            for (int q = 0; q < a.n_save; q++)
-                a.out[((int64_t)q * a.T + tp) * p.P + lane] = read_u(pg, w, __ldg(a.save_idx + q));
-        tp++;
-    }
-    const double h = a.h;
-    const double abstol2 = a.abstol * a.abstol;
-    // a specialised kernel is generated for one integration method: branches on it fold
-    const int amethod = PG::kMethod >= 0 ? PG::kMethod : a.method;
-    // `fresh`: the stamp slots of the nonlinear devices hold their values AT the current iterate.
-    // A step that converged ends with an evaluation at its final u, and the next step starts its
-    // Newton iteration from that same u: G(u), C(u) and the companion currents are functions of
-    // u alone, so the first residual of a step re-assembles them with the new source values and
-    // history terms instead of evaluating every device model again for identical values.
-    bool fresh = false;
-    // Quiescent-step bypass (backward Euler).  `quiet`: the previous step of this lane converged at its first
-    // residual -- no solve, so u == u_n, d == 0 and the stamps are those of u.  If in addition every source stamp
-    // of the new step is bitwise what it was, the new step's first residual F = G u - b is bit for bit the one
-    // that just passed the test: the step would assemble the same numbers, find them converged and change
-    // nothing.  When that holds for all 32 lanes of the warp the step is not executed (its saved point is
-    // written from the unchanged u).  Identical waveforms, statuses and Newton counts by construction; a lane
-    // that could not skip alone executes the step as usual.
-    bool quiet = false;
-    int nexec = 0;                                 // steps this lane executed (not bypassed)
-    for (int64_t k = a.k_begin; k <= a.k_end; k++) {
-        const double t = a.t0 + (double)k * h;
-        const int method = (k == 1) ? CB200_METHOD_BE : amethod;
-        const double gamma = method == CB200_METHOD_BE ? 1.0 / h
-                           : method == CB200_METHOD_TRAP ? 2.0 / h : 3.0 / (2.0 * h);
-@SRC_OLD@
-        eval_sources_step(pg, w, k, k == a.k_begin, a.t0, h, CB200_MODE_TRAN);
-        if (PG::kMethod == CB200_METHOD_BE && !kNlTimeDep) {
-            bool same = quiet && k != a.k_begin;
-@SRC_SAME@
-            if (CB_GROUP_ALL(same)) {
-                if (k % a.save_every == 0 || k == a.nsteps) {
-                    if (act)
-                        for (int q = 0; q < a.n_save; q++)
-                            a.out[((int64_t)q * a.T + tp) * p.P + lane] = read_u(pg, w, __ldg(a.save_idx + q));
-                    tp++;
-                }
-                continue;
-            }
-        }
-        const int solves0 = solves;
-        nexec++;
-        // history terms; un <- u
-        CB_UNROLL
-        for (int i = 0; i < pg.n(); i++) {
-            const double ui = w(pg.off_u() + i);
-            if (method == CB200_METHOD_GEAR2) w(pg.off_dterm() + i) = -(ui - w(pg.off_un() + i)) / (2.0 * h);
-            else if (method == CB200_METHOD_BE) w(pg.off_dterm() + i) = 0.0;
-            /* trap: dterm already holds -du_n */
-            w(pg.off_un() + i) = ui;
-        }
-        bool done = false;
-        int st = CB200_LANE_OK;
-        // a.limit (CB200_TRAN_LIMIT): a step the plain iteration does not finish in max_nl solves
-        // is redone from u_n with the PCNR corrector after every solve (4*max_nl solves allowed)
-        bool lim_on = false;
-        int it0 = 0;
-        for (int it = 0;; it++) {
-            // lanes that are fresh recompute identical values when another lane of the warp is not
-            if (__any_sync(0xffffffffu, kNlTimeDep || !fresh)) { eval_nonlinear(pg, w, t, CB200_MODE_TRAN, false); evals++; }
-            fresh = true;
-            bool bad;
-            const double nrm2 = assemble<true>(pg, lu, w, gamma, sp.gshunt, sp.srcFact, bad);
-            bool restart = false;
-            if (!done) {
-                if (bad) { done = true; st = CB200_LANE_NONFINITE; }
-                else if (nrm2 < abstol2) { done = true; }
-                else if (it - it0 >= (lim_on ? 4 * a.max_nl : a.max_nl)) {
-                    if (PG::kTranLimit && a.limit && !lim_on) { lim_on = true; it0 = it + 1; restart = true; }
-                    else { done = true; st = CB200_LANE_MAXITER; }
-                }
-            }
-            if (CB_GROUP_ALL(done)) break;
-            bool singular;
-            const bool ok = factor_and_solve(pg, lu, w, singular);
-            if (!done) {
-                if (restart) {                             // redo the step from u_n, limiting on
-                    CB_UNROLL
-                    for (int i = 0; i < pg.n(); i++) w(pg.off_u() + i) = w(pg.off_un() + i);
-                    fresh = false;
-                } else if (!ok) { done = true; st = singular ? CB200_LANE_SINGULAR : CB200_LANE_NONFINITE; }
-                else {
-                    apply_update(pg, lu, w);
-                    fresh = false;
-                    solves++;
-                    if (lim_on) {                          // PCNR corrector, solve.jl:686-689
-                        const int lim0 = pg.n() - pg.n_limits();
-                        CB_UNROLL
-                        for (int q = 0; q < pg.n_limits(); q++) w(pg.off_u() + lim0 + q) = w(pg.off_limw() + q);
-                    }
-                }
-            }
-        }
-        quiet = st == CB200_LANE_OK && solves == solves0 && !lim_on;
-        if (st != CB200_LANE_OK && status == CB200_LANE_OK) status = st;
-        if (st != CB200_LANE_OK) fresh = false;           // the last evaluation was not at the state kept
-        if (st == CB200_LANE_NONFINITE || st == CB200_LANE_SINGULAR) {  // dead lane: hold last state
-            CB_UNROLL
-            for (int i = 0; i < pg.n(); i++) w(pg.off_u() + i) = w(pg.off_un() + i);
-        }
-        if (amethod == CB200_METHOD_TRAP) {               // dterm <- -du_{n+1}
-            CB_UNROLL
-            for (int i = 0; i < pg.n(); i++)
-                w(pg.off_dterm() + i) = -(gamma * (w(pg.off_u() + i) - w(pg.off_un() + i)) + w(pg.off_dterm() + i));
-        }
-        if (k % a.save_every == 0 || k == a.nsteps) {
-            if (act)
-                for (int q = 0; q < a.n_save; q++)
-                    a.out[((int64_t)q * a.T + tp) * p.P + lane] = read_u(pg, w, __ldg(a.save_idx + q));
-            tp++;
-        }
-    }
-    if (act) {
-        CB_UNROLL
-        for (int i = 0; i < pg.n(); i++) {
-            a.u[(int64_t)i * p.P + lane] = w(pg.off_u() + i);
-            if (a.hist != nullptr) {                     // history for a resumed segment
-                a.hist[(int64_t)i * p.P + lane] = w(pg.off_un() + i);
-                a.hist[(int64_t)(pg.n() + i) * p.P + lane] = w(pg.off_dterm() + i);
-            }
-        }
-        a.status[lane] = status;
-        if (a.weak && w.weak) a.weak[lane] = 1;
-        a.iters[lane] += solves;
-        if (a.evals != nullptr) a.evals[lane] += evals;
-        if (threadIdx.y == 0) atomicAdd(&cb200_spec_nexec, (unsigned long long)nexec);
-    }
-}
-)CB200";
-
-static std::string spec_tran_body_text(const SpecInput &in)
+// What the quiescent-step bypass of tran_fixed_body needs of one circuit: the b stamp slots of its sources
+// (a snapshot before the step's source evaluation, and the bitwise comparison after it), and the hook that
+// adds a thread's executed steps to cb200_spec_nexec.
+static void emit_bypass(std::ostringstream &o, const SpecInput &in)
 {
     const Program &p = *in.prog;
     std::ostringstream so, ss;
     int q = 0;
     for (int d : *in.src_list)
         for (int b = (*in.dev_bbase)[d]; b < (*in.dev_bbase)[d + 1]; b++, q++) {
-            so << "        const double src_old" << q << " = w(" << p.off_SB + b << ");\n";
-            ss << "            same = same && (w(" << p.off_SB + b << ") == src_old" << q << ");\n";
+            so << "        old[" << q << "] = w(" << p.off_SB + b << ");\n";
+            ss << "        same = same && (w(" << p.off_SB + b << ") == old[" << q << "]);\n";
         }
-    std::string t = kSpecTranFixedBody;
-    auto put = [&t](const std::string &key, const std::string &val) {
-        const size_t at = t.find(key);
-        if (at != std::string::npos) t.replace(at, key.size(), val);
-    };
-    put("@SRC_OLD@\n", so.str());
-    put("@SRC_SAME@\n", ss.str());
-    return t;
-}
-
-// ---------------------------------------------------------------------------
-// Pair mode (small sweeps): TWO warps per 32 lanes.  A lane-per-thread kernel is latency-bound on one
-// warp's dependent chain once a GPU holds fewer lanes than fill it (C3: 12 500 lanes per GPU under
-// 8-way strong scaling run as long as 25 000); most of that chain is the nonlinear device models.  In
-// pair mode a block is dim3(32, 2): both warps carry the SAME 32 lanes with identical register state,
-// each evaluates every second nonlinear device of the lane -- different warps, so the two straight-line
-// model bodies run concurrently instead of one after the other -- and the stamp values cross through
-// shared memory (one [slot][32] row per stamp, two block barriers per Newton iteration).  Everything
-// else (assembly, LU, solves, step control) is computed redundantly by both warps on identical data, so
-// the control flow of the two warps is identical and the results are bit-identical to the single-warp
-// kernel.  Only role 0 accumulates the per-lane counters.  Generated when every nonlinear device is an
-// emitted Verilog-A module (their iterate-dependent pass writes stamp slots and limit-corrector slots only).
-// MEASURED (C3, one B200, profiles/README.md r02r): bit-identical, and SLOWER -- 12 500 lanes 30.4 ms against
-// 15.7 ms, 3 125 lanes 22.9 against 15.4, one lane 8.4 against 6.0: an evaluation pass of ONE body per warp plus
-// the exchange takes twice as long as both bodies in one warp (ptxas: 2072 bytes of spill stack against 408; the
-// 262 exchanged values are all live across the barrier).  So it is opt-in (CB200_PAIR=1), kept for the test
-// that pins its equivalence; the intra-lane parallelism that would pay needs ONE shared model body executed
-// by both threads on per-thread operands (DESIGN.md s. 7).
-struct PairPlan {
-    bool ok = false;
-    std::vector<int> dev[2];       // nonlinear devices of each role
-    std::vector<int> slots[2];     // workspace slots each role's devices write in the iterate-dependent pass
-};
-
-static PairPlan plan_pair(const SpecInput &in)
-{
-    PairPlan pl;
-    const Structure &st = *in.st;
-    const Program &p = *in.prog;
-    if (in.nl_list->size() < 2 || getenv("CB200_NO_PAIR")) return pl;
-    for (int d : *in.nl_list)
-        if ((*in.dev_kind)[d] != CB200_DEV_VA) return pl;
-    const int lim_lo = st.n - st.n_limits;      // limit unknowns: 1-based indices (lim_lo, n]
-    for (size_t q = 0; q < in.nl_list->size(); q++) {
-        const int d = (*in.nl_list)[q], r = (int)(q & 1);
-        pl.dev[r].push_back(d);
-        for (int g = (*in.dev_gbase)[d]; g < (*in.dev_gbase)[d + 1]; g++) pl.slots[r].push_back(p.off_SG + g);
-        for (int c = (*in.dev_cbase)[d]; c < (*in.dev_cbase)[d + 1]; c++) pl.slots[r].push_back(p.off_SC + c);
-        for (int b = (*in.dev_bbase)[d]; b < (*in.dev_bbase)[d + 1]; b++) pl.slots[r].push_back(p.off_SB + b);
-        for (int i = (*in.dev_node_ptr)[d]; i < (*in.dev_node_ptr)[d + 1]; i++) {
-            const int v = (*in.dev_nodes)[i];
-            if (v > lim_lo) pl.slots[r].push_back(p.off_limw + v - 1 - lim_lo);
-        }
-    }
-    pl.ok = true;
-    return pl;
-}
-
-static void emit_pair_program(std::ostringstream &o, const PairPlan &pl)
-{
-    o << "struct SProgP : SProg {\n";
-    o << "    template <typename W>\n    __device__ static __forceinline__ void eval_nonlinear(W &w, double t, int mode, bool initjct)\n    {\n";
-    o << "        SProgP pg;\n        extern __shared__ double cb200_xch[];\n        const int ln = threadIdx.x;\n";
-    const int n0 = (int)pl.slots[0].size();
-    o << "        if (threadIdx.y == 0) {\n";
-    for (int d : pl.dev[0]) o << "            eval_device<1>(pg, w, " << d << ", t, mode, initjct);\n";
-    for (size_t k = 0; k < pl.slots[0].size(); k++)
-        o << "            cb200_xch[" << k * 32 << " + ln] = w(" << pl.slots[0][k] << ");\n";
-    o << "        } else {\n";
-    for (int d : pl.dev[1]) o << "            eval_device<1>(pg, w, " << d << ", t, mode, initjct);\n";
-    for (size_t k = 0; k < pl.slots[1].size(); k++)
-        o << "            cb200_xch[" << (n0 + k) * 32 << " + ln] = w(" << pl.slots[1][k] << ");\n";
-    o << "        }\n        __syncthreads();\n        if (threadIdx.y == 0) {\n";
-    for (size_t k = 0; k < pl.slots[1].size(); k++)
-        o << "            w(" << pl.slots[1][k] << ") = cb200_xch[" << (n0 + k) * 32 << " + ln];\n";
-    o << "        } else {\n";
-    for (size_t k = 0; k < pl.slots[0].size(); k++)
-        o << "            w(" << pl.slots[0][k] << ") = cb200_xch[" << k * 32 << " + ln];\n";
-    o << "        }\n        __syncthreads();\n    }\n};\n";
-    o << "constexpr int kPairSmemBytes = " << (pl.slots[0].size() + pl.slots[1].size()) * 32 * 8 << ";\n";
+    o << "    static constexpr int kSrcSlots = " << q << ";\n";
+    o << "    template <typename W>\n    __device__ static __forceinline__ void src_snapshot(W &w, double *old)\n    {\n"
+      << so.str() << "    }\n";
+    o << "    template <typename W>\n    __device__ static __forceinline__ bool src_same(W &w, const double *old, bool same)\n    {\n"
+      << ss.str() << "        return same;\n    }\n";
+    o << "    __device__ static __forceinline__ void count_steps(int nexec)\n    {\n"
+         "        atomicAdd(&cb200_spec_nexec, (unsigned long long)nexec);\n    }\n";
 }
 
 std::string generate_spec_source(const SpecInput &in)
@@ -469,14 +232,18 @@ std::string generate_spec_source(const SpecInput &in)
     g_prefix = "SProg";
     head << "// generated by cadnip-b200 (specialize.cpp) -- circuit-specialised kernels; do not edit\n";
     if (!in.va_header_path.empty())
-        head << "#define CB200_VA_FN " << (getenv("CB200_SPEC_VA_NOINLINE") ? "__noinline__" : "__forceinline__")
-             << "\n#define CB200_VA_HEADER \"" << in.va_header_path << "\"\n";
-    head << "#include <cstdlib>\n#include \"lane_kernels.cuh\"\n";
+        head << "#define CB200_VA_FN __forceinline__\n#define CB200_VA_HEADER \"" << in.va_header_path << "\"\n";
+    head << "#include \"lane_kernels.cuh\"\n";
     head << "namespace {\nusing namespace cb200;\n";
+    // CB200_NO_BYPASS=1 generates the fixed-step kernel without the quiescent-step bypass of tran_fixed_body
+    const bool bypass = getenv("CB200_NO_BYPASS") == nullptr;
+    if (bypass) o << "__device__ unsigned long long cb200_spec_nexec;   // lane-steps executed (not bypassed) since last read\n";
     o << "struct SProg {\n";
     o << "    static constexpr bool kStatic = true;\n    static constexpr int kUnroll = 4096;\n";
     o << "    static constexpr int kMethod = " << in.method << ";\n";
     o << "    static constexpr bool kTranLimit = " << (in.tran_limit ? "true" : "false") << ";\n";
+    o << "    static constexpr bool kBypass = " << (bypass ? "true" : "false") << ";\n";
+    if (bypass) emit_bypass(o, in);
     emit_const(o, "n", st.n);
     emit_const(o, "n_limits", st.n_limits);
     emit_const(o, "nnz", st.nnz);
@@ -554,26 +321,8 @@ std::string generate_spec_source(const SpecInput &in)
     o << "constexpr int kBlock = " << in.block << ";\nconstexpr int kMinBlocks = " << in.min_blocks << ";\n";
     o << "__global__ void __launch_bounds__(kBlock, kMinBlocks) cb200_spec_dc_kernel(Program p, SpecArgs sp, DcArgs a)\n"
          "{\n    SProg pg; SLuDc lu; RegWs<kSlots> w;\n    dc_body(pg, lu, w, p, sp, a);\n}\n";
-    const bool bypass = getenv("CB200_NO_BYPASS") == nullptr;
-    const char *tran_body = bypass ? "spec_tran_fixed_body" : "tran_fixed_body";
-    // CB200_LOCKSTEP=1: the warps of a block walk the time loop together (block-wide votes, which are barriers):
-    // they then execute the straight-line model bodies at the same time and share instruction fetches -- the
-    // kernel is bound by instruction fetch (profiles/README.md: icc hit rate 73 %, no_instructions 25 %)
-    if (bypass) o << "#define CB_GROUP_ALL(x) " << (getenv("CB200_LOCKSTEP") ? "(__syncthreads_and(x) != 0)" : "__all_sync(0xffffffffu, (x))") << "\n";
-    if (bypass) o << "__device__ unsigned long long cb200_spec_nexec;   // lane-steps executed (not bypassed) since last read\n"
-                  << spec_tran_body_text(in);
     o << "__global__ void __launch_bounds__(kBlock, kMinBlocks) cb200_spec_tran_fixed_kernel(Program p, SpecArgs sp, TranArgs a)\n"
-         "{\n    SProg pg; SLuTr lu; RegWs<kSlots> w;\n    " << tran_body << "(pg, lu, w, p, sp, a);\n}\n";
-    const PairPlan pair = plan_pair(in);
-    if (pair.ok) {
-        emit_pair_program(o, pair);
-        // role 1 computes the same lanes: its read-modify-write counters go to a scratch array
-        o << "__device__ int *cb200_pair_scratch;\n";
-        o << "__global__ void __launch_bounds__(64, 1) cb200_spec_tran_fixed_pair_kernel(Program p, SpecArgs sp, TranArgs a)\n"
-             "{\n    SProgP pg; SLuTr lu; RegWs<kSlots> w;\n"
-             "    if (threadIdx.y != 0) { a.iters = cb200_pair_scratch; a.evals = nullptr; }\n"
-             "    " << tran_body << "(pg, lu, w, p, sp, a);\n}\n";
-    }
+         "{\n    SProg pg; SLuTr lu; RegWs<kSlots> w;\n    tran_fixed_body(pg, lu, w, p, sp, a);\n}\n";
     if (in.with_adaptive)
         o << "__global__ void __launch_bounds__(kBlock, kMinBlocks) cb200_spec_tran_adaptive_kernel(Program p, SpecArgs sp, AdaptArgs a)\n"
              "{\n    SProg pg; SLuTr lu; RegWs<kSlots> w;\n    tran_adaptive_body(pg, lu, w, p, sp, a);\n}\n";
@@ -584,32 +333,10 @@ std::string generate_spec_source(const SpecInput &in)
          "                                     const cb200::DcArgs *a, cudaStream_t st)\n{\n"
          "    const unsigned grid = (unsigned)((p->P + kBlock - 1) / kBlock);\n"
          "    cb200_spec_dc_kernel<<<grid, kBlock, 0, st>>>(*p, *s, *a);\n    return cudaGetLastError();\n}\n";
-    o << "extern \"C\" int cb200_spec_pair_lanes(void);\n";
     o << "extern \"C\" cudaError_t cb200_spec_tran_fixed(const cb200::Program *p, const cb200::SpecArgs *s,\n"
-         "                                             const cb200::TranArgs *a, cudaStream_t st)\n{\n";
-    if (pair.ok)
-        o << "    // pair mode is OPT-IN (CB200_PAIR=1): measured on a B200 it loses to the single-warp kernel at every\n"
-             "    // sweep size (profiles/README.md, r02r)\n"
-             "    static int wave = -1;\n    static int *scratch = nullptr;\n    static int64_t scratch_n = 0;\n"
-             "    if (wave < 0) {\n"
-             "        int dev = 0, sms = 0, nb = 0;\n        cudaGetDevice(&dev);\n"
-             "        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);\n"
-             "        cudaFuncSetAttribute(cb200_spec_tran_fixed_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kPairSmemBytes);\n"
-             "        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, cb200_spec_tran_fixed_pair_kernel, 64, kPairSmemBytes);\n"
-             "        wave = nb * sms * 32;\n    }\n"
-             "    const char *force = getenv(\"CB200_PAIR\");\n"
-             "    const bool use_pair = force && force[0] == '1' && wave > 0;\n"
-             "    if (use_pair) {\n"
-             "        if (scratch_n < p->P) {\n            if (scratch) cudaFree(scratch);\n"
-             "            if (cudaMalloc(&scratch, sizeof(int) * (size_t)p->P) != cudaSuccess) return cudaGetLastError();\n"
-             "            scratch_n = p->P;\n"
-             "            cudaMemcpyToSymbolAsync(cb200_pair_scratch, &scratch, sizeof(int *), 0, cudaMemcpyHostToDevice, st);\n        }\n"
-             "        const unsigned grid = (unsigned)((p->P + 31) / 32);\n"
-             "        cb200_spec_tran_fixed_pair_kernel<<<grid, dim3(32, 2, 1), kPairSmemBytes, st>>>(*p, *s, *a);\n"
-             "        return cudaGetLastError();\n    }\n";
-    o << "    const unsigned grid = (unsigned)((p->P + kBlock - 1) / kBlock);\n"
+         "                                             const cb200::TranArgs *a, cudaStream_t st)\n{\n"
+         "    const unsigned grid = (unsigned)((p->P + kBlock - 1) / kBlock);\n"
          "    cb200_spec_tran_fixed_kernel<<<grid, kBlock, 0, st>>>(*p, *s, *a);\n    return cudaGetLastError();\n}\n";
-    o << "extern \"C\" int cb200_spec_pair_lanes(void) { return " << (pair.ok ? 1 : 0) << "; }\n";
     if (bypass)
         o << "// lane-steps the fixed-step kernels executed since the last call (then reset): the bypass makes it less than\n"
              "// steps x lanes, and the FP64 roofline counts one assembly per EXECUTED step\n"
@@ -671,7 +398,7 @@ void unload_kernel_set(KernelSet &k)
 }
 
 // Cache key of a kernel set: the emitted header, the sources it is rebuilt from, and CB200_NVCC_FLAGS
-// (extra compiler flags for tuning experiments, e.g. -DCB200_WARP_MIN_BLOCKS=8).
+// (extra compiler flags, e.g. -Xptxas -O1).
 static std::string va_kernel_set_keys(const std::string &va_header_text, const std::string &csrc_dir,
                                       std::string &hdr_hex, std::string &so_hex, std::string &extra)
 {

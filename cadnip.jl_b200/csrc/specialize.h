@@ -10,7 +10,7 @@
 
 namespace cb200 {
 
-constexpr int kSpecAbi = 8;
+constexpr int kSpecAbi = 9;
 
 struct SpecInput {
     const Structure *st;

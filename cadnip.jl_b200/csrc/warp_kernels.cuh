@@ -21,10 +21,9 @@
 // are consecutive addresses, a warp's accesses coalesce, and the resident working set
 // (16 warps/SM * 148 SMs * 40 KB = 95 MB) lives in the 126 MB L2.  The arrays on the
 // DEPENDENT chains of the refactor and the triangular solves -- the LU factor, the residual /
-// solution vector, the work vector and the reciprocal pivots (3n + nnz_LU doubles, 9 KB for the
-// flip-flop) -- are staged in SHARED memory (struct Hot): a pivot step is two dependent memory
-// round trips, and at L2 latency those 145 * 2 * 3 round trips were the whole iteration
-// (measured: 3.75 s per C4 sweep with the factor in L2; see profiles/README.md).
+// solution vector, the work vector and the reciprocal pivots -- stay in that row (struct Hot
+// points at them): measured on C4, a copy in shared memory lost to the L1 it takes from the
+// lane rows (DESIGN.md s. 4c).
 #pragma once
 #include "lane_kernels.cuh"
 
@@ -32,16 +31,13 @@ namespace cb200 {
 
 #define CB_FULL 0xffffffffu
 
-// latency-critical arrays of a lane: shared memory when they fit (generic pointers: the same
-// code runs with them left in the lane's global row)
 // The read-only tables the warp kernels walk on every Newton iteration (segment lists, CSR view,
 // level schedule: 43 KB for the flip-flop).  Every data access of the assembly and of the
 // refactor is index -> data, so an index that misses the L1 (the lane rows and the model body's
-// spills compete for it) puts an L2 round trip on the dependent chain.  A block CAN stage the
-// tables in shared memory once (stage_tables, kernels.cu; CB200_WARP_STAGE_TABLES=1) -- measured
-// on C4 that loses (2.00 s vs 1.34 s): the shared memory it takes from the L1 costs more than the
-// guaranteed index hits save -- so by default WTab points at the global arrays.  The struct
-// itself lives in shared memory.
+// spills compete for it) puts an L2 round trip on the dependent chain.  Staging the tables in
+// shared memory once per block was measured on C4 and loses (2.00 s vs 1.34 s): the shared memory
+// it takes from the L1 costs more than the guaranteed index hits save -- so WTab points at the
+// global arrays (stage_tables, kernels.cu).  The struct itself lives in shared memory.
 struct WTab {
     const int *gseg_ptr, *gseg_idx, *cseg_ptr, *cseg_idx, *bseg_ptr, *bseg_idx, *rowptr, *row_nz, *nz_col;
     const int *jmap, *fill_slots, *colperm;
@@ -51,7 +47,7 @@ struct WTab {
 };
 
 struct Hot {
-    double *F, *wv, *DI, *LU;
+    double *F, *wv, *DI, *LU;   // latency-critical arrays of the lane, in its workspace row
     double *buf;      // shared-memory gather buffer of the segmented assembly, ch doubles
     int ch;
     const WTab *tb;   // in shared memory

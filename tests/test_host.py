@@ -251,6 +251,9 @@ def test_emitter_generates_compilable_source(tmp_path):
     assert "cb200_spec_tran_fixed_kernel" in src and "eval_device<1>(pg, w, 2," in src
     assert "__device__ constexpr int k_SProg_dev_node[]" in src      # tables at namespace scope, not on the stack
     assert "__launch_bounds__(kBlock, kMinBlocks)" in src and "constexpr int kMinBlocks = 7;" in src
+    # one time loop (tran_fixed_body of lane_kernels.cuh, with the bypass as a program trait) and one fixed-step kernel
+    assert "static constexpr bool kBypass = true;" in src and "tran_fixed_body(pg, lu, w, p, sp, a);" in src
+    assert "spec_tran_fixed_body" not in src and "pair" not in src
     cu = tmp_path / "spec.cu"
     cu.write_text(src)
     nvcc = backend.nvcc_path()

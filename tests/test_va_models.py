@@ -633,23 +633,20 @@ def test_gpu_va_c3_corner_lanes_with_transient_limiting():
 
 
 @pytest.mark.gpu
-def test_gpu_pair_mode_and_bypass_equal_plain_kernel(monkeypatch):
-    """Three builds of the specialised fixed-step kernel on the C3 corner lanes must agree bit for bit --
+def test_gpu_bypass_equals_plain_kernel(monkeypatch):
+    """Two builds of the specialised fixed-step kernel on the C3 corner lanes must agree bit for bit --
     waveforms, statuses, Newton counts, segmented or not -- and match the oracle: the plain time loop
-    (CB200_NO_BYPASS=1), the default one with the quiescent-step bypass (steps whose first residual would be
-    bitwise the one that just converged are not executed: specialize.cpp, kSpecTranFixedBody), and pair mode
-    (two warps per 32 lanes, one sp_mos1 body each, stamps exchanged through shared memory: plan_pair)."""
+    (CB200_NO_BYPASS=1) and the default one with the quiescent-step bypass (steps whose first residual would be
+    bitwise the one that just converged are not executed: lane_kernels.cuh, tran_fixed_body)."""
     lc = fixture("mos1_c3")
     nl = oracle_of(lc)
     save = [lc.index_of("q"), lc.index_of("d")]
     out = {}
-    for pair in ("plain", "0", "1"):
-        if pair == "plain":
+    for build in ("plain", "bypass"):
+        if build == "plain":
             monkeypatch.setenv("CB200_NO_BYPASS", "1")
-            monkeypatch.setenv("CB200_PAIR", "0")
         else:
             monkeypatch.delenv("CB200_NO_BYPASS", raising=False)
-            monkeypatch.setenv("CB200_PAIR", pair)
         comp = cb.CompiledSweep(lc, cb.MNASpec(mode="tran"))
         try:
             comp.specialize(1e-10, "be", limit=True, fixed_only=True)
@@ -659,21 +656,19 @@ def test_gpu_pair_mode_and_bypass_equal_plain_kernel(monkeypatch):
             host = np.full_like(r["u"], np.nan)
             r3 = comp.tran_fetch((0.0, 1.3e-7), 1e-10, host, method="be", save_idxs=save, save_every=10, limit=True,
                                  n_segments=3)
-            out[pair] = (r["u"], r["status"], r["newton_iters"], r3["u"], r3["newton_iters"], comp.handle.stats())
+            out[build] = (r["u"], r["status"], r["newton_iters"], r3["u"], r3["newton_iters"], comp.handle.stats())
         finally:
             comp.close()
-    for other in ("0", "1"):
-        for a, b in zip(out["plain"][:5], out[other][:5]):
-            assert np.array_equal(a, b, equal_nan=True), other
-    assert out["0"][5]["device_evals"] == out["plain"][5]["device_evals"]
-    assert np.array_equal(out["1"][0], out["1"][3])            # segmented = single launch in pair mode too
+    for a, b in zip(out["plain"][:5], out["bypass"][:5]):
+        assert np.array_equal(a, b, equal_nan=True)
+    assert out["bypass"][5]["device_evals"] == out["plain"][5]["device_evals"]
+    assert np.array_equal(out["bypass"][0], out["bypass"][3])   # segmented = single launch with the bypass
     ro = ora.sweep_tran(nl, ora.make_spec(mode="tran"), 0.0, 1.3e-7,
                         ora.make_tran_opts(method=0, dt=1e-10, save_every=10, limit=True), save)
-    gpu = np.transpose(out["1"][0], (2, 1, 0))
-    assert (out["1"][1] == 0).all() and _close(gpu, ro["u"][:, :gpu.shape[1], :])
-    assert np.array_equal(out["1"][2], ro["newton_iters"])
-    print("kernel ms: plain loop", out["plain"][5]["tran_kernel_ms"], "with bypass", out["0"][5]["tran_kernel_ms"],
-          "pair mode", out["1"][5]["tran_kernel_ms"])
+    gpu = np.transpose(out["bypass"][0], (2, 1, 0))
+    assert (out["bypass"][1] == 0).all() and _close(gpu, ro["u"][:, :gpu.shape[1], :])
+    assert np.array_equal(out["bypass"][2], ro["newton_iters"])
+    print("kernel ms: plain loop", out["plain"][5]["tran_kernel_ms"], "with bypass", out["bypass"][5]["tran_kernel_ms"])
 
 
 @pytest.mark.gpu
