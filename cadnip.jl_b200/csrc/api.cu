@@ -158,18 +158,18 @@ struct DevLu {
 
 }  // namespace
 
+static const int kMaxSegments = 16;      // time segments of a pipelined fixed-step run (cb200_tran_fetch)
+// Lanes per block of the lane-per-thread kernels: at most this many with the workspace in shared memory,
+// this many with it in HBM
+static const int kThreadBlock = 64;
+
 struct cb200_handle {
     int device = 0;
     cudaStream_t stream = nullptr;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
     std::string err;
     Structure st;
-    // host copies of the description
-    std::vector<int> dev_kind, dev_flags, dev_node_ptr, dev_nodes, dev_param_ptr, dev_params;
-    std::vector<int> dev_gbase, dev_cbase, dev_bbase, dev_sbase, src_list, nl_list, limit_init_ref;
-    std::vector<unsigned char> src_uniform;
-    std::vector<double> uniform;
-    int n_lane_cols = 0;
+    Circuit c;                     // host copy of the description
     // lanes
     int64_t P = 0;
     std::vector<double> lanes_host;
@@ -189,7 +189,7 @@ struct cb200_handle {
     DevBuf<int> d_save, d_rejected, d_evals;
     DevBuf<double> d_hist;         // [2n][P] integrator history between time segments
     cudaStream_t copy_stream = nullptr;
-    cudaEvent_t seg_ev[16] = {};
+    cudaEvent_t seg_ev[kMaxSegments] = {};
     std::vector<double> tstops;    // sorted breakpoints for adaptive stepping
     DevBuf<double> d_tstops;
     std::shared_ptr<BufPool> pool;  // recycled waveform buffers (shared with live waves)
@@ -197,14 +197,12 @@ struct cb200_handle {
     DevLu lu[2];                   // 0: DC (gamma = 0), 1: transient
     int lu_gen[2] = {0, 0};        // bumped by every (re-)analysis
     KernelSet k;                   // table-driven kernels: built-in, or rebuilt with VA models
-    bool has_va = false;
     SpecModule spec;               // circuit-specialised kernels (optional)
     int spec_gen[2] = {-1, -1};    // schedule generations the module was generated from
     int spec_method = -1;          // integration method baked into the transient kernel
     bool spec_limit = false;       // transient kernels were generated with the CB200_TRAN_LIMIT path
     int num_sms = 148;
     size_t smem_limit = 0;
-    int block_pref = 64;
     cb200_stats stats{};
     std::vector<cb200_wave *> waves;   // live waves: orphaned (buffers released) by cb200_destroy
 };
@@ -267,9 +265,9 @@ static void layout_workspace(cb200_handle *h)
     p.off_SC = o; o += (int)h->st.nC;
     p.off_SB = o; o += (int)h->st.nb;
     p.off_limw = o; o += h->st.n_limits;
-    p.off_lp = o; o += h->n_lane_cols;
-    p.off_DS = o; o += h->dev_sbase.empty() ? 0 : h->dev_sbase.back();
-    p.off_srcc = o; o += (int)h->src_list.size();
+    p.off_lp = o; o += h->c.n_lane_cols;
+    p.off_DS = o; o += h->c.dev_sbase.empty() ? 0 : h->c.dev_sbase.back();
+    p.off_srcc = o; o += (int)h->c.src_list.size();
     p.off_h1 = o; o += n;
     p.off_h2 = o; o += n;
     p.off_phi = o; o += 6 * n;
@@ -286,11 +284,32 @@ static void layout_workspace(cb200_handle *h)
     p.n_slots_w = (o + 15) / 16 * 16;
 }
 
-// the lane workspace lives in global memory (lane-per-warp kernels, or shared-memory overflow)
-static bool needs_global_ws(const cb200_handle *h)
+// Lane mapping of the table-driven kernels for the handle's program and lane count, and the lanes per block.
+// Lane-per-warp kernels serve the circuits whose lane workspace leaves fewer than 64 lanes per block in
+// shared memory (n_slots > ~450): with one thread per lane such a circuit keeps a few warps per SM busy,
+// each stalled on its own memory column.  Lane-per-block kernels serve LARGE circuits run on few lanes: one
+// warp would evaluate thousands of device instances and walk 1e5 matrix entries alone while 147 SMs idle.
+// CB200_LANE_PER_THREAD=1 keeps the lane-per-thread kernels (A/B parity tests), CB200_LANE_PER_WARP=1 forces
+// the warp kernels, CB200_LANE_PER_BLOCK=1 / =0 forces / forbids the block kernels in their place, and
+// CB200_FORCE_GLOBAL_WS=1 keeps every lane workspace out of shared memory (test hook).
+struct LaneMap {
+    int kind;                      // kernels.h: LaneMapping
+    int block;                     // lanes per block
+};
+static LaneMap lane_map(const cb200_handle *h)
 {
-    return use_warp_kernels(h->prog.n_slots, h->smem_limit, h->block_pref) ||
-           choose_block(h->prog.n_slots, h->smem_limit, h->block_pref) == 0;
+    const Program &p = h->prog;
+    int b = 0;                     // lanes per block whose workspaces fit in shared memory (0: none)
+    if (!getenv("CB200_FORCE_GLOBAL_WS"))
+        for (int c = kThreadBlock; c >= 32 && b == 0; c /= 2)
+            if ((size_t)p.n_slots * c * sizeof(double) <= h->smem_limit) b = c;
+    bool warp = b < kThreadBlock;
+    if (getenv("CB200_LANE_PER_THREAD")) warp = false;
+    else if (getenv("CB200_LANE_PER_WARP")) warp = true;
+    if (!warp) return b > 0 ? LaneMap{kLaneSmem, b} : LaneMap{kLaneHbm, kThreadBlock};
+    bool per_block = (p.n_dev >= 1024 || p.n >= 4096) && p.P <= 1024;
+    if (const char *e = getenv("CB200_LANE_PER_BLOCK")) per_block = atoi(e) != 0;
+    return per_block ? LaneMap{kLaneBlock, 1} : LaneMap{kLaneWarp, kWarpsPerBlock};
 }
 
 // devices whose stamps depend on time only (evaluated once per time step) ...
@@ -300,6 +319,46 @@ static bool is_nonlinear_kind(int kind)
 {
     return kind == CB200_DEV_DIODE || kind == CB200_DEV_DIODECAP || kind == CB200_DEV_SIMPLEMOS ||
            kind == CB200_DEV_VA;
+}
+
+// Reads a description (pattern, stamp maps and device table) into st and c and checks it; returns "" or the
+// error, prefixed with the caller's name.
+static std::string read_circuit(const char *who, const cb200_desc &d, Structure &st, Circuit &c)
+{
+    std::string e = build_structure(d, st);
+    if (!e.empty()) return e;
+    const int nd = d.n_devices;
+    for (int i = 0; i < nd; i++)
+        if (d.dev_kind[i] < 1 || d.dev_kind[i] > CB200_DEV_KIND_MAX) return std::string(who) + ": unknown device kind";
+    c.dev_kind = to_int(d.dev_kind, nd);
+    c.dev_flags = to_int(d.dev_flags, nd);
+    c.dev_node_ptr = to_int(d.dev_node_ptr, nd + 1);
+    c.dev_nodes = to_int(d.dev_nodes, nd ? d.dev_node_ptr[nd] : 0);
+    c.dev_param_ptr = to_int(d.dev_param_ptr, nd + 1);
+    c.dev_params = to_int(d.dev_params, nd ? d.dev_param_ptr[nd] : 0);
+    c.dev_gbase = to_int64(d.dev_gbase, nd + 1);
+    c.dev_cbase = to_int64(d.dev_cbase, nd + 1);
+    c.dev_bbase = to_int64(d.dev_bbase, nd + 1);
+    c.dev_sbase = d.dev_state_ptr ? to_int(d.dev_state_ptr, nd + 1) : std::vector<int>(nd + 1, 0);
+    c.uniform.assign(d.uniform, d.uniform + d.n_uniform);
+    c.limit_init_ref = to_int(d.limit_init_ref, d.n_limits);
+    c.n_lane_cols = d.n_lane_cols;
+    for (int r : c.dev_params)
+        if (r >= d.n_uniform || (r < 0 && ~r >= d.n_lane_cols))
+            return std::string(who) + ": parameter reference out of range";
+    for (int v : c.dev_nodes)
+        if (v < 0 || v > st.n) return std::string(who) + ": device node index out of range";
+    for (int i = 0; i < nd; i++) {
+        c.has_va |= c.dev_kind[i] == CB200_DEV_VA;
+        if (is_source_kind(c.dev_kind[i])) {
+            c.src_list.push_back(i);
+            bool uni = true;
+            for (int q = c.dev_param_ptr[i]; q < c.dev_param_ptr[i + 1]; q++) uni &= c.dev_params[q] >= 0;
+            c.src_uniform.push_back(uni ? 1 : 0);
+        }
+        if (is_nonlinear_kind(c.dev_kind[i])) c.nl_list.push_back(i);
+    }
+    return "";
 }
 
 extern "C" int cb200_abi_version(void) { return CB200_ABI_VERSION; }
@@ -319,7 +378,8 @@ extern "C" int cb200_create(const cb200_desc *d, int32_t device, cb200_handle **
         return fail(nullptr, CB200_ENODEVICE,
                     std::string("cb200_create: no usable CUDA device (there is no CPU fallback): ") +
                         (ce != cudaSuccess ? cudaGetErrorString(ce) : "device ordinal out of range"));
-    cb200_handle *h = new cb200_handle();
+    // every return before the release frees what was built so far
+    std::unique_ptr<cb200_handle, decltype(&cb200_destroy)> h(new cb200_handle(), cb200_destroy);
     h->device = device;
     h->k.eval = cb200_k_eval; h->k.dc = cb200_k_dc;
     h->k.tran_fixed = cb200_k_tran_fixed; h->k.tran_adaptive = cb200_k_tran_adaptive;
@@ -330,69 +390,25 @@ extern "C" int cb200_create(const cb200_desc *d, int32_t device, cb200_handle **
         g_pools.push_back(h->pool);
     }
     ce = cudaSetDevice(device);
-    if (ce != cudaSuccess) { delete h; return fail(nullptr, CB200_ECUDA, cudaGetErrorString(ce)); }
+    if (ce != cudaSuccess) return fail(nullptr, CB200_ECUDA, cudaGetErrorString(ce));
     cudaDeviceProp prop;
     cudaGetDeviceProperties(&prop, device);
-    if (prop.major < 10) {
-        std::string m = "cb200_create: device is sm_" + std::to_string(prop.major) + std::to_string(prop.minor) +
-                        "; this library is built for sm_100a only";
-        delete h;
-        return fail(nullptr, CB200_ENODEVICE, m);
-    }
+    if (prop.major < 10)
+        return fail(nullptr, CB200_ENODEVICE, "cb200_create: device is sm_" + std::to_string(prop.major) +
+                                                  std::to_string(prop.minor) + "; this library is built for sm_100a only");
     h->smem_limit = prop.sharedMemPerBlockOptin;
     h->num_sms = prop.multiProcessorCount;
-    std::string e = build_structure(*d, h->st);
-    if (!e.empty()) { delete h; return fail(nullptr, CB200_EINVAL, e); }
-
-    const int nd = d->n_devices;
-    for (int i = 0; i < nd; i++)
-        if (d->dev_kind[i] < 1 || d->dev_kind[i] > CB200_DEV_KIND_MAX) {
-            delete h;
-            return fail(nullptr, CB200_EINVAL, "cb200_create: unknown device kind");
-        }
-    h->dev_kind = to_int(d->dev_kind, nd);
-    for (int kd : h->dev_kind) h->has_va |= (kd == CB200_DEV_VA);
-    h->dev_flags = to_int(d->dev_flags, nd);
-    h->dev_node_ptr = to_int(d->dev_node_ptr, nd + 1);
-    h->dev_nodes = to_int(d->dev_nodes, nd ? d->dev_node_ptr[nd] : 0);
-    h->dev_param_ptr = to_int(d->dev_param_ptr, nd + 1);
-    h->dev_params = to_int(d->dev_params, nd ? d->dev_param_ptr[nd] : 0);
-    h->dev_gbase = to_int64(d->dev_gbase, nd + 1);
-    h->dev_cbase = to_int64(d->dev_cbase, nd + 1);
-    h->dev_bbase = to_int64(d->dev_bbase, nd + 1);
-    h->dev_sbase = d->dev_state_ptr ? to_int(d->dev_state_ptr, nd + 1) : std::vector<int>(nd + 1, 0);
-    h->uniform.assign(d->uniform, d->uniform + d->n_uniform);
-    h->limit_init_ref = to_int(d->limit_init_ref, d->n_limits);
-    h->n_lane_cols = d->n_lane_cols;
-    for (int r : h->dev_params)
-        if (r >= d->n_uniform || (r < 0 && ~r >= d->n_lane_cols)) {
-            delete h;
-            return fail(nullptr, CB200_EINVAL, "cb200_create: parameter reference out of range");
-        }
-    for (int v : h->dev_nodes)
-        if (v < 0 || v > h->st.n) {
-            delete h;
-            return fail(nullptr, CB200_EINVAL, "cb200_create: device node index out of range");
-        }
-    for (int i = 0; i < nd; i++) {
-        if (is_source_kind(h->dev_kind[i])) {
-            h->src_list.push_back(i);
-            bool uni = true;
-            for (int q = h->dev_param_ptr[i]; q < h->dev_param_ptr[i + 1]; q++) uni &= h->dev_params[q] >= 0;
-            h->src_uniform.push_back(uni ? 1 : 0);
-        }
-        if (is_nonlinear_kind(h->dev_kind[i])) h->nl_list.push_back(i);
-    }
+    std::string e = read_circuit("cb200_create", *d, h->st, h->c);
+    if (!e.empty()) return fail(nullptr, CB200_EINVAL, e);
 
     if (cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking) != cudaSuccess ||
-        cudaEventCreate(&h->ev0) != cudaSuccess || cudaEventCreate(&h->ev1) != cudaSuccess) {
-        delete h;
+        cudaEventCreate(&h->ev0) != cudaSuccess || cudaEventCreate(&h->ev1) != cudaSuccess)
         return fail(nullptr, CB200_ECUDA, "cb200_create: stream/event creation failed");
-    }
     cudaStreamCreateWithFlags(&h->copy_stream, cudaStreamNonBlocking);
     for (auto &e : h->seg_ev) cudaEventCreateWithFlags(&e, cudaEventDisableTiming);
     cudaStream_t s = h->stream;
     const Structure &st = h->st;
+    const Circuit &c = h->c;
     std::vector<unsigned char> nd8(st.nz_is_node_diag.begin(), st.nz_is_node_diag.end());
     // CSR view of the CSC pattern for the row-parallel residual of the lane-per-warp kernels:
     // a counting sort over columns in ascending order leaves every row's entries column-sorted
@@ -407,21 +423,21 @@ extern "C" int cb200_create(const cb200_desc *d, int32_t device, cb200_handle **
                 row_nz[fillp[st.rowval[q]]++] = q;
             }
     }
-    bool ok = h->d_dev_kind.upload(h->dev_kind, s) == cudaSuccess &&
-              h->d_dev_flags.upload(h->dev_flags, s) == cudaSuccess &&
-              h->d_dev_node_ptr.upload(h->dev_node_ptr, s) == cudaSuccess &&
-              h->d_dev_nodes.upload(h->dev_nodes, s) == cudaSuccess &&
-              h->d_dev_param_ptr.upload(h->dev_param_ptr, s) == cudaSuccess &&
-              h->d_dev_params.upload(h->dev_params, s) == cudaSuccess &&
-              h->d_dev_gbase.upload(h->dev_gbase, s) == cudaSuccess &&
-              h->d_dev_cbase.upload(h->dev_cbase, s) == cudaSuccess &&
-              h->d_dev_bbase.upload(h->dev_bbase, s) == cudaSuccess &&
-              h->d_dev_sbase.upload(h->dev_sbase, s) == cudaSuccess &&
-              h->d_src_list.upload(h->src_list, s) == cudaSuccess &&
-              h->d_nl_list.upload(h->nl_list, s) == cudaSuccess &&
-              h->d_src_uniform.upload(h->src_uniform, s) == cudaSuccess &&
-              h->d_limit_init_ref.upload(h->limit_init_ref, s) == cudaSuccess &&
-              h->d_uniform.upload(h->uniform, s) == cudaSuccess &&
+    bool ok = h->d_dev_kind.upload(c.dev_kind, s) == cudaSuccess &&
+              h->d_dev_flags.upload(c.dev_flags, s) == cudaSuccess &&
+              h->d_dev_node_ptr.upload(c.dev_node_ptr, s) == cudaSuccess &&
+              h->d_dev_nodes.upload(c.dev_nodes, s) == cudaSuccess &&
+              h->d_dev_param_ptr.upload(c.dev_param_ptr, s) == cudaSuccess &&
+              h->d_dev_params.upload(c.dev_params, s) == cudaSuccess &&
+              h->d_dev_gbase.upload(c.dev_gbase, s) == cudaSuccess &&
+              h->d_dev_cbase.upload(c.dev_cbase, s) == cudaSuccess &&
+              h->d_dev_bbase.upload(c.dev_bbase, s) == cudaSuccess &&
+              h->d_dev_sbase.upload(c.dev_sbase, s) == cudaSuccess &&
+              h->d_src_list.upload(c.src_list, s) == cudaSuccess &&
+              h->d_nl_list.upload(c.nl_list, s) == cudaSuccess &&
+              h->d_src_uniform.upload(c.src_uniform, s) == cudaSuccess &&
+              h->d_limit_init_ref.upload(c.limit_init_ref, s) == cudaSuccess &&
+              h->d_uniform.upload(c.uniform, s) == cudaSuccess &&
               h->d_gseg_ptr.upload(st.gseg_ptr, s) == cudaSuccess &&
               h->d_gseg_idx.upload(st.gseg_idx, s) == cudaSuccess &&
               h->d_cseg_ptr.upload(st.cseg_ptr, s) == cudaSuccess &&
@@ -434,16 +450,13 @@ extern "C" int cb200_create(const cb200_desc *d, int32_t device, cb200_handle **
               h->d_row_nz.upload(row_nz, s) == cudaSuccess &&
               h->d_nz_col.upload(nz_col, s) == cudaSuccess &&
               h->d_node_diag.upload(nd8, s) == cudaSuccess;
-    if (!ok || cudaStreamSynchronize(s) != cudaSuccess) {
-        std::string m = std::string("cb200_create: upload failed: ") + cudaGetErrorString(cudaGetLastError());
-        cb200_destroy(h);
-        return fail(nullptr, CB200_ECUDA, m);
-    }
+    if (!ok || cudaStreamSynchronize(s) != cudaSuccess)
+        return fail(nullptr, CB200_ECUDA, std::string("cb200_create: upload failed: ") + cudaGetErrorString(cudaGetLastError()));
     Program &p = h->prog;
     p.n = st.n; p.n_nodes = st.n_nodes; p.n_limits = st.n_limits; p.nnz = (int)st.nnz;
-    p.nG = (int)st.nG; p.nC = (int)st.nC; p.nb = (int)st.nb; p.n_dev = nd;
-    p.n_src = (int)h->src_list.size(); p.n_nl = (int)h->nl_list.size();
-    p.n_lane_cols = h->n_lane_cols; p.P = 0;
+    p.nG = (int)st.nG; p.nC = (int)st.nC; p.nb = (int)st.nb; p.n_dev = (int)c.dev_kind.size();
+    p.n_src = (int)c.src_list.size(); p.n_nl = (int)c.nl_list.size();
+    p.n_lane_cols = c.n_lane_cols; p.P = 0;
     p.dev_kind = h->d_dev_kind.p; p.dev_flags = h->d_dev_flags.p;
     p.dev_node_ptr = h->d_dev_node_ptr.p; p.dev_nodes = h->d_dev_nodes.p;
     p.dev_param_ptr = h->d_dev_param_ptr.p; p.dev_params = h->d_dev_params.p;
@@ -457,8 +470,8 @@ extern "C" int cb200_create(const cb200_desc *d, int32_t device, cb200_handle **
     p.bseg_ptr = h->d_bseg_ptr.p; p.bseg_idx = h->d_bseg_idx.p;
     p.colptr = h->d_colptr.p; p.rowval = h->d_rowval.p; p.nz_is_node_diag = h->d_node_diag.p;
     p.rowptr = h->d_rowptr.p; p.row_nz = h->d_row_nz.p; p.nz_col = h->d_nz_col.p;
-    layout_workspace(h);
-    *out = h;
+    layout_workspace(h.get());
+    *out = h.release();
     return CB200_OK;
 }
 
@@ -522,10 +535,12 @@ static int ensure_lane_buffers(cb200_handle *h)
     return CB200_OK;
 }
 
-static int ensure_global_ws(cb200_handle *h)
+// HBM workspace of the mapping m.  Lane-per-thread kernels (and cb200_eval): [n_slots][P padded to the block];
+// lane-per-warp / -block kernels: [P][n_slots_w]
+static int ensure_global_ws(cb200_handle *h, const LaneMap &m)
 {
-    // lane-per-thread kernels: [n_slots][P padded to the block (64)]; lane-per-warp: [P][n_slots_w]
-    const size_t need = (size_t)std::max(h->prog.n_slots, h->prog.n_slots_w) * ((h->P + 63) / 64 * 64);
+    const size_t need = m.kind >= kLaneWarp ? (size_t)h->P * h->prog.n_slots_w
+                                            : (size_t)h->prog.n_slots * ((h->P + m.block - 1) / m.block * m.block);
     if (h->d_ws_global.n < need) CUDA_TRY(h, h->d_ws_global.alloc(need));
     return CB200_OK;
 }
@@ -533,7 +548,7 @@ static int ensure_global_ws(cb200_handle *h)
 extern "C" int cb200_set_lanes(cb200_handle *h, int64_t P, int32_t n_cols, const double *soa)
 {
     if (!h || P <= 0) return fail(h, CB200_EINVAL, "cb200_set_lanes: bad arguments");
-    if (n_cols != h->n_lane_cols) return fail(h, CB200_EINVAL, "cb200_set_lanes: column count differs from the description");
+    if (n_cols != h->c.n_lane_cols) return fail(h, CB200_EINVAL, "cb200_set_lanes: column count differs from the description");
     if (n_cols > 0 && !soa) return fail(h, CB200_EINVAL, "cb200_set_lanes: null SoA");
     cudaSetDevice(h->device);
     // New parameter values: the static pivot order was chosen from magnitudes probed on the OLD
@@ -603,7 +618,7 @@ static int upload_lu(cb200_handle *h, DevLu &L)
 
 static int require_models(cb200_handle *h)
 {
-    if (h->has_va && h->k.va_header_path.empty())
+    if (h->c.has_va && h->k.va_header_path.empty())
         return fail(h, CB200_ESTATE, "the circuit contains Verilog-A devices: call cb200_load_va_models first");
     return CB200_OK;
 }
@@ -620,8 +635,8 @@ static int probe_magnitudes(cb200_handle *h, const cb200_spec *spec, double gamm
     const int ns = (int)std::min<int64_t>(P, 16);
     std::vector<int64_t> sample(ns);
     for (int i = 0; i < ns; i++) sample[i] = ns == 1 ? 0 : (int64_t)((double)i * (double)(P - 1) / (double)(ns - 1));
-    std::vector<double> soa((size_t)h->n_lane_cols * ns);
-    for (int c = 0; c < h->n_lane_cols; c++)
+    std::vector<double> soa((size_t)h->c.n_lane_cols * ns);
+    for (int c = 0; c < h->c.n_lane_cols; c++)
         for (int i = 0; i < ns; i++) soa[(size_t)c * ns + i] = h->lanes_host[(size_t)c * P + sample[i]];
     DevBuf<double> d_soa, d_ws, d_G, d_C;
     CUDA_TRY(h, d_soa.upload(soa, h->stream));
@@ -716,7 +731,7 @@ extern "C" int cb200_eval(cb200_handle *h, const cb200_spec *spec, double t, int
     const int n = h->st.n;
     const int64_t nnz = h->st.nnz;
     h->stats = cb200_stats{};
-    int rc = ensure_global_ws(h);
+    int rc = ensure_global_ws(h, lane_map(h));
     if (rc != CB200_OK) return rc;
     cudaStream_t s = h->stream;
     CUDA_TRY(h, cudaMemsetAsync(h->d_ws_global.p, 0, (size_t)h->prog.n_slots * P * sizeof(double), s));
@@ -764,8 +779,9 @@ struct DcRun {
     float kernel_ms = 0;
 };
 
+// One launch for all lanes; table: on the table-driven kernels even where specialised ones are usable
 static int dc_launch(DcRun &r, int algorithm, const unsigned char *d_active, const double *d_gshunt,
-                     const double *d_srcfact)
+                     const double *d_srcfact, bool table = false)
 {
     cb200_handle *h = r.h;
     DcArgs a{};
@@ -773,17 +789,18 @@ static int dc_launch(DcRun &r, int algorithm, const unsigned char *d_active, con
     a.u = h->d_state.p; a.active = d_active; a.gshunt_lane = d_gshunt; a.srcfact_lane = d_srcfact;
     a.status = h->d_status.p; a.iters = h->d_iters.p; a.converged = h->d_conv.p; a.weak = h->d_weak.p;
     a.ws_global = nullptr;
-    if (needs_global_ws(h)) {
-        int rc = ensure_global_ws(h);
+    const LaneMap m = lane_map(h);
+    if (m.kind != kLaneSmem) {
+        int rc = ensure_global_ws(h, m);
         if (rc != CB200_OK) return rc;
         a.ws_global = h->d_ws_global.p;
     }
     CUDA_TRY(h, cudaEventRecord(h->ev0, h->stream));
-    if (spec_usable(h)) {
+    if (!table && spec_usable(h)) {
         h->stats.launches += 1;
         CUDA_TRY(h, h->spec.dc(&h->prog, &r.sa, &a, h->stream));
     } else {
-        CUDA_TRY(h, h->k.dc(&h->prog, &h->lu[0].prog, &r.sa, &a, h->block_pref, h->smem_limit, h->stream,
+        CUDA_TRY(h, h->k.dc(&h->prog, &h->lu[0].prog, &r.sa, &a, m.kind, m.block, h->smem_limit, h->stream,
                             &h->stats.launches));
     }
     CUDA_TRY(h, cudaEventRecord(h->ev1, h->stream));
@@ -855,22 +872,7 @@ static int dc_chain(cb200_handle *h, const cb200_spec *spec, double t, double ab
         std::vector<int> status01 = status;
         for (int64_t l = 0; l < P; l++) todo[l] = conv[l] ? 0 : 1;
         CUDA_TRY(h, cudaMemcpyAsync(h->d_active.p, todo.data(), P, cudaMemcpyHostToDevice, s));
-        {
-            DcArgs a{};
-            a.algorithm = use_stepping == 3 ? 3 : 2; a.abstol = r.abstol; a.maxiters = r.maxiters; a.t = r.t;
-            a.u = h->d_state.p; a.active = h->d_active.p;
-            a.status = h->d_status.p; a.iters = h->d_iters.p; a.converged = h->d_conv.p; a.weak = h->d_weak.p;
-            if (needs_global_ws(h)) {
-                if ((rc = ensure_global_ws(h)) != CB200_OK) return rc;
-                a.ws_global = h->d_ws_global.p;
-            }
-            CUDA_TRY(h, cudaEventRecord(h->ev0, s));
-            CUDA_TRY(h, h->k.dc(&h->prog, &h->lu[0].prog, &r.sa, &a, h->block_pref, h->smem_limit, s, &h->stats.launches));
-            CUDA_TRY(h, cudaEventRecord(h->ev1, s));
-            CUDA_TRY(h, cudaStreamSynchronize(s));
-            float ms = 0; cudaEventElapsedTime(&ms, h->ev0, h->ev1);
-            r.kernel_ms += ms;
-        }
+        if ((rc = dc_launch(r, use_stepping == 3 ? 3 : 2, h->d_active.p, nullptr, nullptr, true)) != CB200_OK) return rc;
         if ((rc = fetch()) != CB200_OK) return rc;
         h->stats.dc_stepping_lanes = 0;
         for (int64_t l = 0; l < P; l++) {
@@ -930,7 +932,168 @@ extern "C" int cb200_dc(cb200_handle *h, const cb200_spec *spec, const cb200_dc_
 // ---------------------------------------------------------------------------
 // transient
 // ---------------------------------------------------------------------------
-static const int kMaxSegments = 16;
+static double gamma_of(int method, double dt)
+{
+    return (method == CB200_METHOD_BE || method == CB200_METHOD_BDF ? 1.0 : method == CB200_METHOD_TRAP ? 2.0 : 1.5) / dt;
+}
+
+// What the launches of one transient share
+struct TranRun {
+    cb200_handle *h;
+    const cb200_tran_opts *o;
+    SpecArgs sa;
+    LaneMap m;                 // of the table-driven kernels
+    double *ws_global;         // their workspace in HBM, or null
+    double t0, t1;
+    int n_save;
+};
+
+// A fixed-step launch over steps 1..nsteps from the handle's state
+static TranArgs fixed_args(const TranRun &r, int method, double dt, int64_t nsteps, int save_every, int n_save,
+                           int64_t T, double *out)
+{
+    cb200_handle *h = r.h;
+    TranArgs a{};
+    a.method = method; a.t0 = r.t0; a.h = dt; a.nsteps = nsteps; a.k_begin = 1; a.k_end = nsteps;
+    a.abstol = r.o->abstol; a.max_nl = r.o->max_nl_iters; a.limit = r.o->flags & CB200_TRAN_LIMIT;
+    a.save_every = save_every; a.n_save = n_save; a.save_idx = h->d_save.p; a.T = T;
+    a.u = h->d_state.p; a.out = out; a.status = h->d_status.p; a.iters = h->d_iters.p;
+    a.evals = h->d_evals.p; a.weak = h->d_weak.p; a.ws_global = r.ws_global;
+    return a;
+}
+
+// Fixed-step run in time segments, one launch each.  With a host destination the D2H copy of a finished
+// segment runs on the copy stream while the next segment computes.
+static int tran_fixed_run(const TranRun &r, cb200_wave &w, double *host_u, int64_t host_ld, int n_segments)
+{
+    cb200_handle *h = r.h;
+    const cb200_tran_opts *o = r.o;
+    const int64_t P = h->P;
+    const int n = h->st.n, n_save = r.n_save;
+    cudaStream_t s = h->stream;
+    const int64_t nsteps = (int64_t)std::llround((r.t1 - r.t0) / o->dt);
+    const int se = o->save_every > 0 ? o->save_every : 1;
+    const int64_t T = 1 + nsteps / se + ((nsteps % se) ? 1 : 0);
+    w.T = T; w.nsteps = nsteps; w.save_every = se;
+    if (w.d_out.alloc((size_t)std::max(1, n_save) * T * P) != cudaSuccess)
+        return fail(h, CB200_ENOMEM, "cb200_tran: waveform buffer allocation failed");
+    TranArgs a = fixed_args(r, o->method, o->dt, nsteps, se, n_save, T, w.d_out.p);
+    int nseg = (host_u != nullptr && n_segments > 1) ? (int)std::min<int64_t>(n_segments, std::max<int64_t>(1, nsteps / 64)) : 1;
+    if (nseg > kMaxSegments) nseg = kMaxSegments;
+    if (nseg > 1) {
+        if (h->d_hist.n != (size_t)2 * n * P && h->d_hist.alloc((size_t)2 * n * P) != cudaSuccess)
+            return fail(h, CB200_ENOMEM, "cb200_tran: history buffer allocation failed");
+        a.hist = h->d_hist.p;
+    }
+    const int64_t seg_len = (nsteps + nseg - 1) / nseg;
+    bool used_spec = false;            // the launches went to the circuit-specialised kernels
+    cudaError_t ce = cudaSuccess;
+    cudaEventRecord(h->ev0, s);
+    for (int g = 0; g < nseg && ce == cudaSuccess; g++) {
+        a.k_begin = (int64_t)g * seg_len + 1;
+        a.k_end = std::min<int64_t>(nsteps, (int64_t)(g + 1) * seg_len);
+        if (a.k_begin > a.k_end) break;
+        a.tp_begin = g == 0 ? 0 : 1 + (a.k_begin - 1) / se;
+        if (spec_usable(h) && h->spec_method == o->method && (!a.limit || h->spec_limit)) {
+            h->stats.launches += 1;
+            if (!used_spec && h->spec.take_counters) h->spec.take_counters(nullptr, s);   // reset
+            used_spec = true;
+            ce = h->spec.tran_fixed(&h->prog, &r.sa, &a, s);
+        } else {
+            ce = h->k.tran_fixed(&h->prog, &h->lu[1].prog, &r.sa, &a, r.m.kind, r.m.block, h->smem_limit, s,
+                                 &h->stats.launches);
+        }
+        if (host_u != nullptr && ce == cudaSuccess) {
+            int64_t tp_end = 1 + a.k_end / se;                     // one past the last point written
+            if (a.k_end == nsteps && nsteps % se != 0) tp_end += 1;
+            cudaEventRecord(h->seg_ev[g], s);
+            cudaStreamWaitEvent(h->copy_stream, h->seg_ev[g], 0);
+            for (int q = 0; q < n_save; q++) {
+                // host rows may be wider than the device rows (host_ld >= P): this handle's lanes
+                // are then one column block of a waveform array that several GPUs fill
+                const size_t off = ((size_t)q * T + a.tp_begin) * P;
+                const size_t hoff = ((size_t)q * T + a.tp_begin) * (size_t)host_ld;
+                ce = cudaMemcpy2DAsync(host_u + hoff, (size_t)host_ld * sizeof(double), w.d_out.p + off,
+                                       (size_t)P * sizeof(double), (size_t)P * sizeof(double),
+                                       (size_t)(tp_end - a.tp_begin), cudaMemcpyDeviceToHost, h->copy_stream);
+                if (ce != cudaSuccess) break;
+            }
+            h->stats.d2h_bytes += (int64_t)n_save * (tp_end - a.tp_begin) * P * sizeof(double);
+        }
+    }
+    cudaEventRecord(h->ev1, s);
+    if (host_u != nullptr && ce == cudaSuccess) ce = cudaStreamSynchronize(h->copy_stream);
+    if (ce == cudaSuccess) ce = cudaStreamSynchronize(s);
+    if (ce != cudaSuccess) return fail(h, CB200_ECUDA, std::string("cb200_tran: kernel failed: ") + cudaGetErrorString(ce));
+    h->stats.steps_accepted = nsteps * P;
+    if (used_spec && h->spec.take_counters) {
+        // specialised kernels skip quiescent steps bit-exactly (lane_kernels.cuh, tran_fixed_body): the
+        // lane-steps actually executed
+        unsigned long long nexec = 0;
+        if (h->spec.take_counters(&nexec, s) == cudaSuccess) h->stats.steps_accepted = (int64_t)nexec;
+    }
+    return CB200_OK;
+}
+
+// LTE-controlled stepping, per-lane time axis; tstops come from cb200_set_tstops
+static int tran_adaptive_run(const TranRun &r, cb200_wave &w)
+{
+    cb200_handle *h = r.h;
+    const cb200_tran_opts *o = r.o;
+    const int64_t P = h->P;
+    cudaStream_t s = h->stream;
+    const int T = o->max_points > 1 ? o->max_points : 4096;
+    w.T = T;
+    const double span = r.t1 - r.t0;
+    AdaptArgs a{};
+    a.method = o->method == CB200_METHOD_BE ? CB200_METHOD_BE : o->method == CB200_METHOD_BDF ? CB200_METHOD_BDF : CB200_METHOD_TRAP;
+    a.t0 = r.t0; a.t1 = r.t1;
+    a.dtmax = o->dtmax > 0 ? o->dtmax : span / 50.0;
+    a.dtmin = o->dtmin > 0 ? o->dtmin : span * 1e-12;
+    a.h0 = std::min(o->dt, a.dtmax);
+    a.abstol = o->abstol; a.reltol = o->reltol; a.lte_abstol = o->lte_abstol;
+    const bool cls = (o->flags & CB200_TRAN_CLASS_ABSTOL) != 0;
+    a.tol_v = cls ? o->vntol : o->lte_abstol; a.tol_i = cls ? o->iabstol : o->lte_abstol;
+    a.tol_q = cls ? o->chgtol : o->lte_abstol;
+    a.cls_i0 = h->st.n_nodes; a.cls_q0 = h->st.n_nodes + h->st.n_currents;
+    a.cls_l0 = h->st.n_nodes + h->st.n_currents + h->st.n_charges;
+    if (cls && !(a.tol_v > 0 && a.tol_i > 0 && a.tol_q > 0))
+        return fail(h, CB200_EINVAL, "cb200_tran: CB200_TRAN_CLASS_ABSTOL needs vntol, iabstol, chgtol > 0");
+    a.max_nl = o->max_nl_iters; a.limit = o->flags & CB200_TRAN_LIMIT;
+    a.n_save = r.n_save; a.save_idx = h->d_save.p; a.max_points = T;
+    if (w.d_out.alloc((size_t)std::max(1, r.n_save) * T * P) != cudaSuccess ||
+        w.d_t.alloc((size_t)T * P) != cudaSuccess || w.d_count.alloc(P) != cudaSuccess ||
+        (h->d_rejected.n != (size_t)P && h->d_rejected.alloc(P) != cudaSuccess))
+        return fail(h, CB200_ENOMEM, "cb200_tran: waveform buffer allocation failed");
+    a.tstops = h->d_tstops.p; a.n_tstops = (int)h->tstops.size();
+    a.u = h->d_state.p; a.out_t = w.d_t.p; a.out = w.d_out.p; a.count = w.d_count.p;
+    a.status = h->d_status.p; a.iters = h->d_iters.p; a.rejected = h->d_rejected.p;
+    a.evals = h->d_evals.p; a.weak = h->d_weak.p;
+    a.ws_global = r.ws_global;
+    cudaError_t ce;
+    cudaEventRecord(h->ev0, s);
+    if (spec_usable(h) && h->spec.tran_adaptive && h->spec_method == a.method && (!a.limit || h->spec_limit)) {
+        h->stats.launches += 1;
+        ce = h->spec.tran_adaptive(&h->prog, &r.sa, &a, s);
+    } else {
+        ce = h->k.tran_adaptive(&h->prog, &h->lu[1].prog, &r.sa, &a, r.m.kind, r.m.block, h->smem_limit, s,
+                                &h->stats.launches);
+    }
+    cudaEventRecord(h->ev1, s);
+    if (ce == cudaSuccess) {
+        std::vector<int> cnt(P), rj(P);
+        cudaMemcpyAsync(cnt.data(), w.d_count.p, P * sizeof(int), cudaMemcpyDeviceToHost, s);
+        cudaMemcpyAsync(rj.data(), h->d_rejected.p, P * sizeof(int), cudaMemcpyDeviceToHost, s);
+        ce = cudaStreamSynchronize(s);
+        int64_t acc = 0, rejt = 0;
+        for (int64_t l = 0; l < P; l++) { acc += cnt[l] - 1; rejt += rj[l]; }
+        h->stats.steps_accepted = acc;
+        h->stats.steps_rejected = rejt;
+    }
+    if (ce == cudaSuccess) ce = cudaStreamSynchronize(s);
+    if (ce != cudaSuccess) return fail(h, CB200_ECUDA, std::string("cb200_tran: kernel failed: ") + cudaGetErrorString(ce));
+    return CB200_OK;
+}
 
 static int tran_impl(cb200_handle *h, const cb200_spec *spec, double t0, double t1,
                      const cb200_tran_opts *o, const int64_t *save_idx, int32_t n_save,
@@ -972,170 +1135,48 @@ static int tran_impl(cb200_handle *h, const cb200_spec *spec, double t0, double 
         }
         CUDA_TRY(h, cudaMemsetAsync(h->d_iters.p, 0, P * sizeof(int), s));
     }
-    const double gamma_nom = (o->method == CB200_METHOD_BE || o->method == CB200_METHOD_BDF ? 1.0 : o->method == CB200_METHOD_TRAP ? 2.0 : 1.5) / o->dt;
-    int rc = ensure_lu(h, spec, 1, gamma_nom);
+    int rc = ensure_lu(h, spec, 1, gamma_of(o->method, o->dt));
     if (rc != CB200_OK) return rc;
 
-    bool used_spec = false;            // the fixed-step launches went to the circuit-specialised kernels
-    cb200_wave *w = new cb200_wave();
+    std::unique_ptr<cb200_wave> w(new cb200_wave());
     w->h = h; w->P = P; w->n_save = n_save; w->n = n; w->adaptive = o->adaptive; w->t0 = t0; w->dt = o->dt;
     w->d_out.pool = w->d_t.pool = w->d_final.pool = h->pool;
     w->d_count.pool = w->d_status.pool = w->d_iters.pool = h->pool;
     std::vector<int> save0(n_save);
     for (int q = 0; q < n_save; q++) save0[q] = (int)save_idx[q] - 1;
     DevBuf<int> &d_save = h->d_save;
-    if (d_save.n != (size_t)n_save && d_save.alloc(n_save) != cudaSuccess) { delete w; return fail(h, CB200_ECUDA, "cb200_tran: allocation failed"); }
-    if (n_save > 0 && cudaMemcpyAsync(d_save.p, save0.data(), n_save * sizeof(int), cudaMemcpyHostToDevice, s) != cudaSuccess) {
-        delete w; return fail(h, CB200_ECUDA, "cb200_tran: upload failed");
-    }
+    if (d_save.n != (size_t)n_save && d_save.alloc(n_save) != cudaSuccess) return fail(h, CB200_ECUDA, "cb200_tran: allocation failed");
+    if (n_save > 0 && cudaMemcpyAsync(d_save.p, save0.data(), n_save * sizeof(int), cudaMemcpyHostToDevice, s) != cudaSuccess)
+        return fail(h, CB200_ECUDA, "cb200_tran: upload failed");
     // lanes whose initialisation failed keep that status (InitialFailure, dcop.jl:197-200)
-    if (cudaMemcpyAsync(h->d_status.p, st0.data(), P * sizeof(int), cudaMemcpyHostToDevice, s) != cudaSuccess) {
-        delete w; return fail(h, CB200_ECUDA, "cb200_tran: upload failed");
-    }
-    SpecArgs sa = spec_args(spec);
-    sa.mode = CB200_MODE_TRAN;
+    if (cudaMemcpyAsync(h->d_status.p, st0.data(), P * sizeof(int), cudaMemcpyHostToDevice, s) != cudaSuccess)
+        return fail(h, CB200_ECUDA, "cb200_tran: upload failed");
+    TranRun r{h, o, spec_args(spec), lane_map(h), nullptr, t0, t1, n_save};
+    r.sa.mode = CB200_MODE_TRAN;
     if ((h->d_evals.n != (size_t)P && h->d_evals.alloc(P) != cudaSuccess) ||
-        cudaMemsetAsync(h->d_evals.p, 0, P * sizeof(int), s) != cudaSuccess) {
-        delete w; return fail(h, CB200_ECUDA, "cb200_tran: allocation failed");
+        cudaMemsetAsync(h->d_evals.p, 0, P * sizeof(int), s) != cudaSuccess)
+        return fail(h, CB200_ECUDA, "cb200_tran: allocation failed");
+    if (r.m.kind != kLaneSmem) {
+        rc = ensure_global_ws(h, r.m);
+        if (rc != CB200_OK) return rc;
+        r.ws_global = h->d_ws_global.p;
     }
-    double *ws_global = nullptr;
-    if (needs_global_ws(h)) {
-        rc = ensure_global_ws(h);
-        if (rc != CB200_OK) { delete w; return rc; }
-        ws_global = h->d_ws_global.p;
-    }
-    cudaError_t ce = cudaSuccess;
     if (o->init == 2 && o->uic_steps > 0) {
         // CedarUICOp (dcop.jl:311-411): uic_steps backward-Euler steps of uic_dt from the start state
         // on the table-driven kernels (same pivot schedule), nothing saved; Newton failures are
         // marched through (force_dtmin=true), so the lane status is reset afterwards.
         DevBuf<double> scratch;
         scratch.pool = h->pool;
-        if (scratch.alloc((size_t)2 * P) != cudaSuccess) { delete w; return fail(h, CB200_ENOMEM, "cb200_tran: allocation failed"); }
-        TranArgs a{};
-        a.method = CB200_METHOD_BE; a.t0 = t0; a.h = o->uic_dt > 0 ? o->uic_dt : 1e-12; a.nsteps = o->uic_steps;
-        a.k_begin = 1; a.k_end = o->uic_steps; a.tp_begin = 0;
-        a.abstol = o->abstol; a.max_nl = o->max_nl_iters; a.limit = o->flags & CB200_TRAN_LIMIT;
-        a.save_every = o->uic_steps; a.n_save = 0; a.save_idx = d_save.p; a.T = 2;
-        a.u = h->d_state.p; a.out = scratch.p; a.status = h->d_status.p; a.iters = h->d_iters.p;
-        a.evals = h->d_evals.p; a.weak = h->d_weak.p; a.ws_global = ws_global;
-        ce = h->k.tran_fixed(&h->prog, &h->lu[1].prog, &sa, &a, h->block_pref, h->smem_limit, s, &h->stats.launches);
+        if (scratch.alloc((size_t)2 * P) != cudaSuccess) return fail(h, CB200_ENOMEM, "cb200_tran: allocation failed");
+        const TranArgs a = fixed_args(r, CB200_METHOD_BE, o->uic_dt > 0 ? o->uic_dt : 1e-12, o->uic_steps,
+                                      o->uic_steps, 0, 2, scratch.p);
+        cudaError_t ce = h->k.tran_fixed(&h->prog, &h->lu[1].prog, &r.sa, &a, r.m.kind, r.m.block, h->smem_limit, s,
+                                         &h->stats.launches);
         if (ce == cudaSuccess) ce = cudaMemsetAsync(h->d_status.p, 0, P * sizeof(int), s);
-        if (ce != cudaSuccess) { delete w; return fail(h, CB200_ECUDA, std::string("cb200_tran: warm-up failed: ") + cudaGetErrorString(ce)); }
+        if (ce != cudaSuccess) return fail(h, CB200_ECUDA, std::string("cb200_tran: warm-up failed: ") + cudaGetErrorString(ce));
     }
-    if (!o->adaptive) {
-        const int64_t nsteps = (int64_t)std::llround((t1 - t0) / o->dt);
-        const int se = o->save_every > 0 ? o->save_every : 1;
-        const int64_t T = 1 + nsteps / se + ((nsteps % se) ? 1 : 0);
-        w->T = T; w->nsteps = nsteps; w->save_every = se;
-        if (w->d_out.alloc((size_t)std::max(1, n_save) * T * P) != cudaSuccess) {
-            delete w; return fail(h, CB200_ENOMEM, "cb200_tran: waveform buffer allocation failed");
-        }
-        TranArgs a{};
-        a.method = o->method; a.t0 = t0; a.h = o->dt; a.nsteps = nsteps; a.abstol = o->abstol;
-        a.max_nl = o->max_nl_iters; a.limit = o->flags & CB200_TRAN_LIMIT; a.save_every = se; a.n_save = n_save; a.save_idx = d_save.p;
-        a.T = T; a.u = h->d_state.p; a.out = w->d_out.p; a.status = h->d_status.p; a.iters = h->d_iters.p;
-        a.evals = h->d_evals.p; a.weak = h->d_weak.p;
-        a.ws_global = ws_global;
-        // Time segments: one launch each.  With a host destination the D2H copy of a finished
-        // segment runs on the copy stream while the next segment computes.
-        int nseg = (host_u != nullptr && n_segments > 1) ? (int)std::min<int64_t>(n_segments, std::max<int64_t>(1, nsteps / 64)) : 1;
-        if (nseg > kMaxSegments) nseg = kMaxSegments;
-        if (nseg > 1) {
-            if (h->d_hist.n != (size_t)2 * n * P && h->d_hist.alloc((size_t)2 * n * P) != cudaSuccess) {
-                delete w; return fail(h, CB200_ENOMEM, "cb200_tran: history buffer allocation failed");
-            }
-            a.hist = h->d_hist.p;
-        }
-        const int64_t seg_len = (nsteps + nseg - 1) / nseg;
-        cudaEventRecord(h->ev0, s);
-        for (int g = 0; g < nseg && ce == cudaSuccess; g++) {
-            a.k_begin = (int64_t)g * seg_len + 1;
-            a.k_end = std::min<int64_t>(nsteps, (int64_t)(g + 1) * seg_len);
-            if (a.k_begin > a.k_end) break;
-            a.tp_begin = g == 0 ? 0 : 1 + (a.k_begin - 1) / se;
-            if (spec_usable(h) && h->spec_method == o->method && (!a.limit || h->spec_limit)) {
-                h->stats.launches += 1;
-                if (!used_spec && h->spec.take_counters) h->spec.take_counters(nullptr, s);   // reset
-                used_spec = true;
-                ce = h->spec.tran_fixed(&h->prog, &sa, &a, s);
-            } else {
-                ce = h->k.tran_fixed(&h->prog, &h->lu[1].prog, &sa, &a, h->block_pref, h->smem_limit, s, &h->stats.launches);
-            }
-            if (host_u != nullptr && ce == cudaSuccess) {
-                int64_t tp_end = 1 + a.k_end / se;                     // one past the last point written
-                if (a.k_end == nsteps && nsteps % se != 0) tp_end += 1;
-                cudaEventRecord(h->seg_ev[g], s);
-                cudaStreamWaitEvent(h->copy_stream, h->seg_ev[g], 0);
-                for (int q = 0; q < n_save; q++) {
-                    // host rows may be wider than the device rows (host_ld >= P): this handle's lanes
-                    // are then one column block of a waveform array that several GPUs fill
-                    const size_t off = ((size_t)q * T + a.tp_begin) * P;
-                    const size_t hoff = ((size_t)q * T + a.tp_begin) * (size_t)host_ld;
-                    ce = cudaMemcpy2DAsync(host_u + hoff, (size_t)host_ld * sizeof(double), w->d_out.p + off,
-                                           (size_t)P * sizeof(double), (size_t)P * sizeof(double),
-                                           (size_t)(tp_end - a.tp_begin), cudaMemcpyDeviceToHost, h->copy_stream);
-                    if (ce != cudaSuccess) break;
-                }
-                h->stats.d2h_bytes += (int64_t)n_save * (tp_end - a.tp_begin) * P * sizeof(double);
-            }
-        }
-        cudaEventRecord(h->ev1, s);
-        if (host_u != nullptr && ce == cudaSuccess) ce = cudaStreamSynchronize(h->copy_stream);
-    } else {
-        // LTE-controlled stepping, per-lane time axis; tstops come from cb200_set_tstops
-        const int T = o->max_points > 1 ? o->max_points : 4096;
-        w->T = T;
-        const double span = t1 - t0;
-        AdaptArgs a{};
-        a.method = o->method == CB200_METHOD_BE ? CB200_METHOD_BE : o->method == CB200_METHOD_BDF ? CB200_METHOD_BDF : CB200_METHOD_TRAP;
-        a.t0 = t0; a.t1 = t1;
-        a.dtmax = o->dtmax > 0 ? o->dtmax : span / 50.0;
-        a.dtmin = o->dtmin > 0 ? o->dtmin : span * 1e-12;
-        a.h0 = std::min(o->dt, a.dtmax);
-        a.abstol = o->abstol; a.reltol = o->reltol; a.lte_abstol = o->lte_abstol;
-        const bool cls = (o->flags & CB200_TRAN_CLASS_ABSTOL) != 0;
-        a.tol_v = cls ? o->vntol : o->lte_abstol; a.tol_i = cls ? o->iabstol : o->lte_abstol;
-        a.tol_q = cls ? o->chgtol : o->lte_abstol;
-        a.cls_i0 = h->st.n_nodes; a.cls_q0 = h->st.n_nodes + h->st.n_currents;
-        a.cls_l0 = h->st.n_nodes + h->st.n_currents + h->st.n_charges;
-        if (cls && !(a.tol_v > 0 && a.tol_i > 0 && a.tol_q > 0)) { delete w; return fail(h, CB200_EINVAL, "cb200_tran: CB200_TRAN_CLASS_ABSTOL needs vntol, iabstol, chgtol > 0"); }
-        a.max_nl = o->max_nl_iters; a.limit = o->flags & CB200_TRAN_LIMIT;
-        a.n_save = n_save; a.save_idx = d_save.p; a.max_points = T;
-        if (w->d_out.alloc((size_t)std::max(1, n_save) * T * P) != cudaSuccess ||
-            w->d_t.alloc((size_t)T * P) != cudaSuccess || w->d_count.alloc(P) != cudaSuccess ||
-            (h->d_rejected.n != (size_t)P && h->d_rejected.alloc(P) != cudaSuccess)) {
-            delete w; return fail(h, CB200_ENOMEM, "cb200_tran: waveform buffer allocation failed");
-        }
-        a.tstops = h->d_tstops.p; a.n_tstops = (int)h->tstops.size();
-        a.u = h->d_state.p; a.out_t = w->d_t.p; a.out = w->d_out.p; a.count = w->d_count.p;
-        a.status = h->d_status.p; a.iters = h->d_iters.p; a.rejected = h->d_rejected.p;
-        a.evals = h->d_evals.p; a.weak = h->d_weak.p;
-        a.ws_global = ws_global;
-        cudaEventRecord(h->ev0, s);
-        if (spec_usable(h) && h->spec.tran_adaptive && h->spec_method == a.method && (!a.limit || h->spec_limit)) {
-            h->stats.launches += 1;
-            ce = h->spec.tran_adaptive(&h->prog, &sa, &a, s);
-        } else {
-            ce = h->k.tran_adaptive(&h->prog, &h->lu[1].prog, &sa, &a, h->block_pref, h->smem_limit, s, &h->stats.launches);
-        }
-        cudaEventRecord(h->ev1, s);
-        if (ce == cudaSuccess) {
-            std::vector<int> cnt(P), rj(P);
-            cudaMemcpyAsync(cnt.data(), w->d_count.p, P * sizeof(int), cudaMemcpyDeviceToHost, s);
-            cudaMemcpyAsync(rj.data(), h->d_rejected.p, P * sizeof(int), cudaMemcpyDeviceToHost, s);
-            ce = cudaStreamSynchronize(s);
-            int64_t acc = 0, rejt = 0;
-            for (int64_t l = 0; l < P; l++) { acc += cnt[l] - 1; rejt += rj[l]; }
-            h->stats.steps_accepted = acc;
-            h->stats.steps_rejected = rejt;
-        }
-    }
-    if (ce == cudaSuccess) ce = cudaStreamSynchronize(s);
-    if (ce != cudaSuccess) {
-        delete w;
-        return fail(h, CB200_ECUDA, std::string("cb200_tran: kernel failed: ") + cudaGetErrorString(ce));
-    }
+    rc = o->adaptive ? tran_adaptive_run(r, *w) : tran_fixed_run(r, *w, host_u, host_ld, n_segments);
+    if (rc != CB200_OK) return rc;
     float ms = 0; cudaEventElapsedTime(&ms, h->ev0, h->ev1);
     h->stats.kernel_ms += ms;
     h->stats.tran_kernel_ms = ms;
@@ -1144,15 +1185,8 @@ static int tran_impl(cb200_handle *h, const cb200_spec *spec, double t0, double 
     cudaMemcpyAsync(w->d_status.p, h->d_status.p, P * sizeof(int), cudaMemcpyDeviceToDevice, s);
     cudaMemcpyAsync(w->d_iters.p, h->d_iters.p, P * sizeof(int), cudaMemcpyDeviceToDevice, s);
     cudaMemcpyAsync(w->d_final.p, h->d_state.p, (size_t)n * P * sizeof(double), cudaMemcpyDeviceToDevice, s);
-    ce = cudaStreamSynchronize(s);
-    if (ce != cudaSuccess) { delete w; return fail(h, CB200_ECUDA, cudaGetErrorString(ce)); }
-    if (!o->adaptive) h->stats.steps_accepted = w->nsteps * P;
-    if (!o->adaptive && used_spec && h->spec.take_counters) {
-        // specialised kernels skip quiescent steps bit-exactly (lane_kernels.cuh, tran_fixed_body): the
-        // lane-steps actually executed
-        unsigned long long nexec = 0;
-        if (h->spec.take_counters(&nexec, s) == cudaSuccess) h->stats.steps_accepted = (int64_t)nexec;
-    }
+    cudaError_t ce = cudaStreamSynchronize(s);
+    if (ce != cudaSuccess) return fail(h, CB200_ECUDA, cudaGetErrorString(ce));
     {   // device-model evaluation passes executed (sum over lanes): the work the FP64 roofline counts
         std::vector<int> ev(P);
         cudaMemcpyAsync(ev.data(), h->d_evals.p, P * sizeof(int), cudaMemcpyDeviceToHost, s);
@@ -1161,8 +1195,8 @@ static int tran_impl(cb200_handle *h, const cb200_spec *spec, double t0, double 
         for (int64_t l = 0; l < P; l++) tot += ev[l];
         h->stats.device_evals = tot;
     }
-    h->waves.push_back(w);
-    *out = w;
+    h->waves.push_back(w.get());
+    *out = w.release();
     return CB200_OK;
 }
 
@@ -1249,15 +1283,9 @@ extern "C" int cb200_set_tstops(cb200_handle *h, const double *tstops, int32_t n
 static SpecInput spec_input(const cb200_handle &h, int method, int64_t P, int num_sms)
 {
     SpecInput in{};
-    in.st = &h.st; in.prog = &h.prog;
-    in.dev_kind = &h.dev_kind; in.dev_flags = &h.dev_flags; in.dev_node_ptr = &h.dev_node_ptr;
-    in.dev_nodes = &h.dev_nodes; in.dev_param_ptr = &h.dev_param_ptr; in.dev_params = &h.dev_params;
-    in.dev_gbase = &h.dev_gbase; in.dev_cbase = &h.dev_cbase; in.dev_bbase = &h.dev_bbase; in.dev_sbase = &h.dev_sbase;
-    in.src_list = &h.src_list; in.nl_list = &h.nl_list; in.limit_init_ref = &h.limit_init_ref;
-    in.src_uniform = &h.src_uniform; in.method = method;
+    in.st = &h.st; in.prog = &h.prog; in.c = &h.c; in.method = method;
     in.va_header_path = h.k.va_header_path;
-    in.uniform = &h.uniform; in.lu_dc = &h.lu[0].host; in.lu_tr = &h.lu[1].host;
-    in.n_lane_cols = h.n_lane_cols;
+    in.lu_dc = &h.lu[0].host; in.lu_tr = &h.lu[1].host;
     in.block = 64;
     const int64_t lanes_per_sm = (P + num_sms - 1) / num_sms;
     in.min_blocks = std::max(1, std::min((int)((lanes_per_sm + in.block - 1) / in.block), 1024 / in.block));
@@ -1271,7 +1299,7 @@ extern "C" int cb200_specialize(cb200_handle *h, const cb200_spec *spec, int32_t
                                 const char *csrc_dir, const char *cache_dir, int32_t flags)
 {
     if (method < 0 || method > 3 || !(dt > 0.0)) return fail(h, CB200_EINVAL, "cb200_specialize: bad method / dt");
-    const double gamma = (method == CB200_METHOD_BE || method == CB200_METHOD_BDF ? 1.0 : method == CB200_METHOD_TRAP ? 2.0 : 1.5) / dt;
+    const double gamma = gamma_of(method, dt);
     if (!h || !spec || !csrc_dir || !cache_dir) return fail(h, CB200_EINVAL, "cb200_specialize: null argument");
     if (h->P <= 0) return fail(h, CB200_ESTATE, "cb200_specialize: call cb200_set_lanes first");
     cudaSetDevice(h->device);
@@ -1373,9 +1401,7 @@ static int host_lu_check_impl(const cb200_desc *d, const double *absJ, const dou
 extern "C" int cb200_lane_mapping(const cb200_handle *h)
 {
     if (!h) return CB200_EINVAL;
-    if (use_block_kernels(h->prog, h->smem_limit, h->block_pref)) return 3;
-    if (use_warp_kernels(h->prog.n_slots, h->smem_limit, h->block_pref)) return 2;
-    return choose_block(h->prog.n_slots, h->smem_limit, h->block_pref) == 0 ? 1 : 0;
+    return lane_map(h).kind;
 }
 
 // Host-only view of the emitter (no device needed): structure + LU analysis from
@@ -1386,29 +1412,8 @@ extern "C" int64_t cb200_emit_source(const cb200_desc *d, const double *absJ_dc,
 {
     if (!d || !absJ_dc || !absJ_tr) { g_last_error = "cb200_emit_source: null argument"; return CB200_EINVAL; }
     cb200_handle h;
-    std::string e = build_structure(*d, h.st);
+    std::string e = read_circuit("cb200_emit_source", *d, h.st, h.c);
     if (!e.empty()) { g_last_error = e; return CB200_EINVAL; }
-    const int nd = d->n_devices;
-    h.dev_kind = to_int(d->dev_kind, nd); h.dev_flags = to_int(d->dev_flags, nd);
-    h.dev_node_ptr = to_int(d->dev_node_ptr, nd + 1);
-    h.dev_nodes = to_int(d->dev_nodes, nd ? d->dev_node_ptr[nd] : 0);
-    h.dev_param_ptr = to_int(d->dev_param_ptr, nd + 1);
-    h.dev_params = to_int(d->dev_params, nd ? d->dev_param_ptr[nd] : 0);
-    h.dev_gbase = to_int64(d->dev_gbase, nd + 1); h.dev_cbase = to_int64(d->dev_cbase, nd + 1);
-    h.dev_bbase = to_int64(d->dev_bbase, nd + 1);
-    h.dev_sbase = d->dev_state_ptr ? to_int(d->dev_state_ptr, nd + 1) : std::vector<int>(nd + 1, 0);
-    h.uniform.assign(d->uniform, d->uniform + d->n_uniform);
-    h.limit_init_ref = to_int(d->limit_init_ref, d->n_limits);
-    h.n_lane_cols = d->n_lane_cols;
-    for (int i = 0; i < nd; i++) {
-        if (is_source_kind(h.dev_kind[i])) {
-            h.src_list.push_back(i);
-            bool uni = true;
-            for (int q = h.dev_param_ptr[i]; q < h.dev_param_ptr[i + 1]; q++) uni &= h.dev_params[q] >= 0;
-            h.src_uniform.push_back(uni ? 1 : 0);
-        }
-        if (is_nonlinear_kind(h.dev_kind[i])) h.nl_list.push_back(i);
-    }
     std::vector<double> a0(absJ_dc, absJ_dc + h.st.nnz), a1(absJ_tr, absJ_tr + h.st.nnz);
     e = analyze_lu(h.st, a0, 1e-3, h.lu[0].host);
     if (e.empty()) e = analyze_lu(h.st, a1, 1e-3, h.lu[1].host);
@@ -1619,7 +1624,7 @@ extern "C" int cb200_flop_model(const cb200_handle *h, int64_t *out)
         out[2 + w] = fac; out[4 + w] = sol;
     }
     out[6] = st.n;
-    out[7] = (int64_t)h->nl_list.size();
+    out[7] = (int64_t)h->c.nl_list.size();
     return CB200_OK;
 }
 

@@ -29,6 +29,19 @@ struct Structure {
 // Build pattern and maps from resolved 1-based COO.  Returns "" or an error.
 std::string build_structure(const cb200_desc &d, Structure &out);
 
+// Host copy of the device table of a checked description (api.cu: read_circuit), and the device
+// lists derived from it.
+struct Circuit {
+    std::vector<int> dev_kind, dev_flags, dev_node_ptr, dev_nodes, dev_param_ptr, dev_params;
+    std::vector<int> dev_gbase, dev_cbase, dev_bbase, dev_sbase, limit_init_ref;
+    std::vector<double> uniform;
+    int n_lane_cols = 0;
+    std::vector<int> src_list;               // devices whose stamps depend on t only (sources)
+    std::vector<unsigned char> src_uniform;  // [src] 1: every parameter of the source is uniform
+    std::vector<int> nl_list;                // devices whose stamps depend on the iterate
+    bool has_va = false;
+};
+
 // Static-pivot sparse LU schedule (the symbolic phase that replaces KLU analyze).
 struct LuSchedule {
     int n = 0;

@@ -95,8 +95,6 @@ struct DcArgs {
     double *ws_global;      // used when the lane workspace does not fit in shared memory
     int gather_ch;          // set by the launcher: doubles of the shared-memory gather buffer of a lane-per-warp / -block lane
 };
-cudaError_t launch_dc(const Program &p, const LuProgram &lu, const SpecArgs &s, const DcArgs &a,
-                      int block, size_t smem_limit, cudaStream_t st, int64_t *launches);
 
 // ---- transient, fixed step (BE / trap / Gear-2), whole time loop on the device
 struct TranArgs {
@@ -122,9 +120,6 @@ struct TranArgs {
     double *ws_global;
     int gather_ch;
 };
-cudaError_t launch_tran_fixed(const Program &p, const LuProgram &lu, const SpecArgs &s,
-                              const TranArgs &a, int block, size_t smem_limit, cudaStream_t st,
-                              int64_t *launches);
 
 // ---- transient, adaptive (trap + LTE), per-lane time axis
 struct AdaptArgs {
@@ -152,18 +147,15 @@ struct AdaptArgs {
     double *ws_global;
     int gather_ch;
 };
-cudaError_t launch_tran_adaptive(const Program &p, const LuProgram &lu, const SpecArgs &s,
-                                 const AdaptArgs &a, int block, size_t smem_limit,
-                                 cudaStream_t st, int64_t *launches);
 
 cudaError_t launch_debug_exp(const double *x, double *y, int n, cudaStream_t st);
 
-// pick lanes-per-block so the lane workspace fits in shared memory (0 = use global)
-int choose_block(int n_slots, size_t smem_limit, int preferred);
-// true: the circuit runs on the lane-per-warp kernels (workspace [lane][n_slots_w] in HBM / L2)
-bool use_warp_kernels(int n_slots, size_t smem_limit, int preferred);
-// true: ... on the lane-per-BLOCK kernels (large circuits on few lanes)
-bool use_block_kernels(const Program &p, size_t smem_limit, int preferred);
+// Lane mapping of the table-driven kernels (cb200_lane_mapping), chosen by api.cu; the launchers take it
+// with the lanes per block.  Lane-per-thread kernels: workspace [n_slots][lanes] in shared memory (0) or
+// in HBM (1); lane-per-warp (2) and lane-per-block (3): workspace row [lane][n_slots_w] in HBM.
+enum LaneMapping { kLaneSmem = 0, kLaneHbm = 1, kLaneWarp = 2, kLaneBlock = 3 };
+constexpr int kWarpsPerBlock = 16;       // lanes of a lane-per-warp block (one per SM: the warps share one WTab)
+constexpr int kKernelSetAbi = 3;         // cb200_k_abi() of a kernel set with these launchers
 
 }  // namespace cb200
 
@@ -173,10 +165,10 @@ int cb200_k_abi(void);
 cudaError_t cb200_k_eval(const cb200::Program *, const cb200::SpecArgs *, const cb200::EvalArgs *,
                          cudaStream_t, int64_t *);
 cudaError_t cb200_k_dc(const cb200::Program *, const cb200::LuProgram *, const cb200::SpecArgs *,
-                       const cb200::DcArgs *, int, size_t, cudaStream_t, int64_t *);
+                       const cb200::DcArgs *, int, int, size_t, cudaStream_t, int64_t *);
 cudaError_t cb200_k_tran_fixed(const cb200::Program *, const cb200::LuProgram *, const cb200::SpecArgs *,
-                               const cb200::TranArgs *, int, size_t, cudaStream_t, int64_t *);
+                               const cb200::TranArgs *, int, int, size_t, cudaStream_t, int64_t *);
 cudaError_t cb200_k_tran_adaptive(const cb200::Program *, const cb200::LuProgram *,
-                                  const cb200::SpecArgs *, const cb200::AdaptArgs *, int, size_t,
+                                  const cb200::SpecArgs *, const cb200::AdaptArgs *, int, int, size_t,
                                   cudaStream_t, int64_t *);
 }

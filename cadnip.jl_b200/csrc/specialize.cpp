@@ -207,10 +207,11 @@ static void emit_lu(std::ostringstream &o, const char *sname, const Structure &s
 static void emit_bypass(std::ostringstream &o, const SpecInput &in)
 {
     const Program &p = *in.prog;
+    const Circuit &c = *in.c;
     std::ostringstream so, ss;
     int q = 0;
-    for (int d : *in.src_list)
-        for (int b = (*in.dev_bbase)[d]; b < (*in.dev_bbase)[d + 1]; b++, q++) {
+    for (int d : c.src_list)
+        for (int b = c.dev_bbase[d]; b < c.dev_bbase[d + 1]; b++, q++) {
             so << "        old[" << q << "] = w(" << p.off_SB + b << ");\n";
             ss << "        same = same && (w(" << p.off_SB + b << ") == old[" << q << "]);\n";
         }
@@ -227,6 +228,7 @@ std::string generate_spec_source(const SpecInput &in)
 {
     const Structure &st = *in.st;
     const Program &p = *in.prog;
+    const Circuit &c = *in.c;
     std::ostringstream head, data, o;
     g_data = &data;
     g_prefix = "SProg";
@@ -247,28 +249,28 @@ std::string generate_spec_source(const SpecInput &in)
     emit_const(o, "n", st.n);
     emit_const(o, "n_limits", st.n_limits);
     emit_const(o, "nnz", st.nnz);
-    emit_const(o, "n_dev", (long long)in.dev_kind->size());
-    emit_const(o, "n_src", (long long)in.src_list->size());
-    emit_const(o, "n_nl", (long long)in.nl_list->size());
-    emit_const(o, "n_lane_cols", in.n_lane_cols);
-    emit_int_table(o, "src_list", *in.src_list);
-    emit_int_table(o, "nl_list", *in.nl_list);
-    emit_int_table(o, "dev_kind", *in.dev_kind);
-    emit_int_table(o, "dev_flags", *in.dev_flags);
-    emit_int_table(o, "dev_node_ptr", *in.dev_node_ptr);
-    emit_int_table(o, "dev_node", *in.dev_nodes);
-    emit_int_table(o, "dev_param_ptr", *in.dev_param_ptr);
-    emit_int_table(o, "dev_param", *in.dev_params);
-    emit_int_table(o, "dev_gbase", *in.dev_gbase);
-    emit_int_table(o, "dev_cbase", *in.dev_cbase);
-    emit_int_table(o, "dev_bbase", *in.dev_bbase);
-    emit_int_table(o, "dev_sbase", *in.dev_sbase);
+    emit_const(o, "n_dev", (long long)c.dev_kind.size());
+    emit_const(o, "n_src", (long long)c.src_list.size());
+    emit_const(o, "n_nl", (long long)c.nl_list.size());
+    emit_const(o, "n_lane_cols", c.n_lane_cols);
+    emit_int_table(o, "src_list", c.src_list);
+    emit_int_table(o, "nl_list", c.nl_list);
+    emit_int_table(o, "dev_kind", c.dev_kind);
+    emit_int_table(o, "dev_flags", c.dev_flags);
+    emit_int_table(o, "dev_node_ptr", c.dev_node_ptr);
+    emit_int_table(o, "dev_node", c.dev_nodes);
+    emit_int_table(o, "dev_param_ptr", c.dev_param_ptr);
+    emit_int_table(o, "dev_param", c.dev_params);
+    emit_int_table(o, "dev_gbase", c.dev_gbase);
+    emit_int_table(o, "dev_cbase", c.dev_cbase);
+    emit_int_table(o, "dev_bbase", c.dev_bbase);
+    emit_int_table(o, "dev_sbase", c.dev_sbase);
     data << "__device__ constexpr double k_SProg_uniform[] = {";
-    if (in.uniform->empty()) data << "0.0";
-    for (size_t i = 0; i < in.uniform->size(); i++) data << (i ? "," : "") << hexdouble((*in.uniform)[i]);
+    if (c.uniform.empty()) data << "0.0";
+    for (size_t i = 0; i < c.uniform.size(); i++) data << (i ? "," : "") << hexdouble(c.uniform[i]);
     data << "};\n";
     o << "    __device__ static constexpr double uniform(int i) { return k_SProg_uniform[i]; }\n";
-    emit_int_table(o, "limit_init_ref", *in.limit_init_ref);
+    emit_int_table(o, "limit_init_ref", c.limit_init_ref);
     emit_int_table(o, "gseg_ptr", st.gseg_ptr);
     emit_int_table(o, "gseg_idx", st.gseg_idx);
     emit_int_table(o, "cseg_ptr", st.cseg_ptr);
@@ -300,19 +302,19 @@ std::string generate_spec_source(const SpecInput &in)
     emit_accumulate(o, st, p);
     // straight-line device evaluation lists (eval_all / eval_nonlinear / eval_sources)
     o << "    template <typename W>\n    __device__ static __forceinline__ void eval_all(W &w, double t, int mode, bool initjct)\n    {\n        SProg pg;\n";
-    for (size_t d = 0; d < in.dev_kind->size(); d++)
+    for (size_t d = 0; d < c.dev_kind.size(); d++)
         o << "        eval_device<0>(pg, w, " << d << ", t, mode, initjct);\n";
     o << "    }\n";
     o << "    template <typename W>\n    __device__ static __forceinline__ void eval_nonlinear(W &w, double t, int mode, bool initjct)\n    {\n        SProg pg;\n";
-    for (int d : *in.nl_list) o << "        eval_device<1>(pg, w, " << d << ", t, mode, initjct);\n";
+    for (int d : c.nl_list) o << "        eval_device<1>(pg, w, " << d << ", t, mode, initjct);\n";
     o << "    }\n";
     o << "    template <typename W>\n    __device__ static __forceinline__ void eval_sources(W &w, double t, int mode)\n    {\n        SProg pg;\n";
-    for (int d : *in.src_list) o << "        eval_device<2>(pg, w, " << d << ", t, mode, false);\n";
+    for (int d : c.src_list) o << "        eval_device<2>(pg, w, " << d << ", t, mode, false);\n";
     o << "    }\n";
     o << "    template <typename W>\n    __device__ static __forceinline__ void eval_sources_step(W &w, int64_t k, bool first, double t0, double h, int mode)\n    {\n        SProg pg;\n";
-    for (size_t q = 0; q < in.src_list->size(); q++)
-        o << "        source_step_one(pg, w, " << q << ", " << (*in.src_list)[q] << ", "
-          << ((*in.src_uniform)[q] ? "true" : "false") << ", k, first, t0, h, mode);\n";
+    for (size_t q = 0; q < c.src_list.size(); q++)
+        o << "        source_step_one(pg, w, " << q << ", " << c.src_list[q] << ", "
+          << (c.src_uniform[q] ? "true" : "false") << ", k, first, t0, h, mode);\n";
     o << "    }\n";
     o << "};\n";
     emit_lu(o, "SLuDc", st, p, *in.lu_dc);
@@ -464,11 +466,13 @@ std::string build_va_kernel_set(const std::string &va_header_text, const std::st
     }
     void *dl = open_module(so);
     if (!dl) return std::string("va models: dlopen failed: ") + dlerror();
+    typedef int (*int_fn)(void);
+    int_fn abi = (int_fn)dlsym(dl, "cb200_k_abi");
     out.eval = (k_eval_fn)dlsym(dl, "cb200_k_eval");
     out.dc = (k_dc_fn)dlsym(dl, "cb200_k_dc");
     out.tran_fixed = (k_tran_fn)dlsym(dl, "cb200_k_tran_fixed");
     out.tran_adaptive = (k_adapt_fn)dlsym(dl, "cb200_k_tran_adaptive");
-    if (!out.eval || !out.dc || !out.tran_fixed || !out.tran_adaptive) {
+    if (!abi || !out.eval || !out.dc || !out.tran_fixed || !out.tran_adaptive || abi() != kKernelSetAbi) {
         out = KernelSet();
         return "va models: " + so + " does not export the kernel entry points";
     }

@@ -15,16 +15,12 @@ constexpr int kSpecAbi = 9;
 struct SpecInput {
     const Structure *st;
     const Program *prog;              // workspace offsets / n_slots
-    const std::vector<int> *dev_kind, *dev_flags, *dev_node_ptr, *dev_nodes, *dev_param_ptr,
-        *dev_params, *dev_gbase, *dev_cbase, *dev_bbase, *dev_sbase, *src_list, *nl_list, *limit_init_ref;
-    const std::vector<double> *uniform;
-    const std::vector<unsigned char> *src_uniform;
+    const Circuit *c;
     int method;                       // CB200_METHOD_* compiled into the transient kernel
     std::string va_header_path;       // emitted Verilog-A models ("" = none)
     bool with_adaptive = true;        // also generate the adaptive transient kernel (a third of the compile time)
     bool tran_limit = false;          // compile the CB200_TRAN_LIMIT restart path into the transient kernels
     const LuSchedule *lu_dc, *lu_tr;
-    int n_lane_cols;
     int block, min_blocks;            // __launch_bounds__ of the generated kernels
 };
 
@@ -46,11 +42,11 @@ struct SpecModule {
 // A kernel set: the table-driven kernels of kernels.cu, either the library's built-in
 // copy or a variant rebuilt with Verilog-A device models (-DCB200_VA_HEADER=...).
 typedef cudaError_t (*k_eval_fn)(const Program *, const SpecArgs *, const EvalArgs *, cudaStream_t, int64_t *);
-typedef cudaError_t (*k_dc_fn)(const Program *, const LuProgram *, const SpecArgs *, const DcArgs *, int,
+typedef cudaError_t (*k_dc_fn)(const Program *, const LuProgram *, const SpecArgs *, const DcArgs *, int, int,
                                size_t, cudaStream_t, int64_t *);
-typedef cudaError_t (*k_tran_fn)(const Program *, const LuProgram *, const SpecArgs *, const TranArgs *, int,
+typedef cudaError_t (*k_tran_fn)(const Program *, const LuProgram *, const SpecArgs *, const TranArgs *, int, int,
                                  size_t, cudaStream_t, int64_t *);
-typedef cudaError_t (*k_adapt_fn)(const Program *, const LuProgram *, const SpecArgs *, const AdaptArgs *, int,
+typedef cudaError_t (*k_adapt_fn)(const Program *, const LuProgram *, const SpecArgs *, const AdaptArgs *, int, int,
                                   size_t, cudaStream_t, int64_t *);
 struct KernelSet {
     void *dl = nullptr;

@@ -268,6 +268,23 @@ def test_emitter_generates_compilable_source(tmp_path):
     assert max(frames) <= 64, frames
 
 
+def test_emitter_rejects_unknown_device_kind():
+    """cb200_emit_source checks the description as cb200_create does: no source for a device kind
+    the kernels do not know."""
+    import dataclasses
+    from cadnip_b200.workloads import clipper_sweep
+    cs = clipper_sweep(2, 1)
+    params, P = cs.lane_params()
+    lc = cb.lower(cs.builder, params, cb.MNASpec(mode="tran"), P=P)
+    kind = np.array(lc.dev_kind, dtype=np.int32)
+    kind[1] = 1000
+    bad = dataclasses.replace(lc, dev_kind=kind)
+    assert "cb200_spec_tran_fixed_kernel" in backend.emit_source(lc, np.ones(1 << 12), np.ones(1 << 12))
+    with pytest.raises(backend.CB200Error) as e:
+        backend.emit_source(bad, np.ones(1 << 12), np.ones(1 << 12))
+    assert e.value.code == backend.EINVAL and "unknown device kind" in str(e.value)
+
+
 def _random_matrix_on_pattern(colptr, rowval, rng):
     """Random values on a CSC pattern (1-based), made safely non-singular: strong diagonal where the
     pattern has one, O(1) couplings elsewhere (MNA source rows have a structurally zero diagonal)."""
